@@ -21,6 +21,12 @@ factors with the distributed result. The previous round's workload (weak-scaled 
 --impl reference: times the CPU restatement of the reference's algorithm (oracle/, OpenMP over the host cores; faer itself
 needs a Rust toolchain that this image does not have) — LLT at the SAME n = 16384 at N = 1, a bounded sample of the LU at
 N > 1 (the port needs ~80 s for one n = 32768 factorisation).
+
+--dump-outputs DIR (N = 1 GPU arm): after the timed steps, writes the Cholesky factor the last timed step left in A as
+float64 .npy files, so that two builds can be compared output for output on the same seeded input:
+  llt_factor_diagonal.npy  the n diagonal entries of L
+  llt_factor_columns.npy   n x k: L's columns at k sorted indices drawn by numpy's default_rng(0) (all columns when they fit),
+                           entries above the diagonal (not part of the factor) set to 0; k * n * 8 <= 32 MiB
 """
 from __future__ import annotations
 
@@ -324,6 +330,22 @@ def run_lu(torch, dist, lay, lib, dev, stream, world, rank, local_rank, n, nb, s
     return out
 
 
+DUMP_COLUMN_BYTES = 32 << 20  # sampled columns of the factor written by --dump-outputs
+
+
+def dump_llt_factor(torch, A, out_dir: str) -> None:
+    """Writes the diagonal and a fixed, seeded sample of columns of the lower-triangular factor held in A (see --dump-outputs)."""
+    n = A.shape[0]
+    k = min(n, max(1, DUMP_COLUMN_BYTES // (8 * n)))
+    cols = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+    idx = torch.as_tensor(cols, device=A.device)
+    rows = torch.arange(n, device=A.device)
+    L = torch.where(rows[:, None] >= idx[None, :], A[:, idx], torch.zeros((), dtype=A.dtype, device=A.device))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "llt_factor_diagonal.npy"), torch.diagonal(A).cpu().numpy())
+    np.save(os.path.join(out_dir, "llt_factor_columns.npy"), L.cpu().numpy())
+
+
 DIST_NB = 1024
 LU_NB = 512   # block-column width of the LU runs (configs[2])
 
@@ -484,7 +506,13 @@ def main():
     ap.add_argument("--nb", type=int, default=DIST_NB, help="block-column width of the distributed layout (N>1)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the factor of the last one as DIR/<name>.npy (1-GPU arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.gpus != 1):
+        ap.error("--dump-outputs needs the 1-GPU arm (--impl b200 --gpus 1)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     if args.impl == "reference":
@@ -573,6 +601,8 @@ def main():
     ms_per_step = ms_total / args.steps
     # one factorisation of the (global) n x n matrix per step, whatever the number of ranks
     value = llt_flops(n) / (ms_per_step * 1e-3) / 1e12
+    if args.dump_outputs:
+        dump_llt_factor(torch, A, args.dump_outputs)
 
     # ---- correctness guard on the timed data (cheap probe): A x == L (L^T x), reduced over the ranks ----
     torch.manual_seed(99)

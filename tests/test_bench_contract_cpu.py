@@ -27,6 +27,13 @@ def test_reference_arm_prints_one_contract_line():
     assert "workload" in d["config"]
 
 
+def test_bench_rejects_zero_steps_and_dumps_outside_the_gpu_arm():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "dump"], ["--gpus", "2", "--dump-outputs", "dump"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=120,
+                             cwd=ROOT)
+        assert out.returncode == 2 and "error:" in out.stderr, (extra, out.stderr[-2000:])
+
+
 def test_non_zero_ranks_of_the_reference_arm_exit_quietly():
     env = dict(os.environ)
     env["RANK"] = "1"; env["WORLD_SIZE"] = "2"
