@@ -377,22 +377,6 @@ void lu_rec_cx(cudaStream_t st, View<R> A, i64 start, i64 end, int* trans) {
   swap_cols(csub(A, 0, end, m, ncols - end));
 }
 
-// dst (compact column-major complex, ld = nrows) [i, c] = src[perm[i], c]
-template <class R>
-__global__ void gather_rows_cx_kernel(R* __restrict__ dst, const R* __restrict__ src, i64 rs, i64 cs, i64 nrows,
-                                       const long long* __restrict__ perm) {
-  const i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x;
-  const i64 c = blockIdx.y;
-  if (i < nrows) cst(dst, c * nrows + i, cld(src, perm[i] * rs + c * cs));
-}
-template <class R>
-__global__ void scatter_rows_cx_kernel(R* __restrict__ dst, i64 rs, i64 cs, const R* __restrict__ src, i64 nrows) {
-  const i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x;
-  const i64 c = blockIdx.y;
-  if (i < nrows) cst(dst, i * rs + c * cs, cld(src, c * nrows + i));
-}
-
-
 // conj?(T) X = rhs, T lower / upper triangular (unit diagonal or not); views in complex units
 template <class R>
 void solve_lower_triangular_in_place_cx(cudaStream_t st, View<const R> tril, bool unit, bool conj, View<R> rhs) {
@@ -471,25 +455,10 @@ size_t lu_partial_piv_in_place_cx(cudaStream_t st, View<R> A, long long* perm_fw
   return n_trans;
 }
 
-// rhs[i, :] <- rhs[perm[i], :] (perm: HOST int64 of length nrows) through a compact copy
+// a complex-unit view as a view of (re, im) elements, for the element-generic row permutation of solve_f64.cu; ReIm<R> keeps R's
+// alignment, so a device rhs aligned only to sizeof(R) is moved as before
 template <class R>
-void permute_rows_cx(cudaStream_t st, View<R> rhs, const long long* perm) {
-  const i64 n = rhs.nrows, k = rhs.ncols;
-  if (n == 0 || k == 0) return;
-  FB_ASSERT(k < 65536, "too many right-hand sides for one permutation launch");
-  long long* d_perm = (long long*)ws_alloc((size_t)n * 8);
-  R* tmp = (R*)ws_alloc((size_t)n * (size_t)k * 2 * sizeof(R));
-  FB_CUDA_CHECK(cudaMemcpyAsync(d_perm, perm, (size_t)n * 8, cudaMemcpyHostToDevice, st));
-  dim3 grid((unsigned)((n + 255) / 256), (unsigned)k);
-  gather_rows_cx_kernel<R><<<grid, 256, 0, st>>>(tmp, rhs.ptr, rhs.rs, rhs.cs, n, d_perm);
-  scatter_rows_cx_kernel<R><<<grid, 256, 0, st>>>(rhs.ptr, rhs.rs, rhs.cs, tmp, n);
-  FB_CUDA_CHECK(cudaGetLastError());
-  note_launch();
-  note_launch();
-  FB_CUDA_CHECK(cudaStreamSynchronize(st));
-  ws_free(tmp);
-  ws_free(d_perm);
-}
+View<ReIm<R>> as_pairs(View<R> v) { return View<ReIm<R>>{(ReIm<R>*)v.ptr, v.nrows, v.ncols, v.rs, v.cs}; }
 
 // rhs <- conj?(A)^-1 rhs from the factors (lu/partial_pivoting/solve.rs:21-54): permute rows, unit-lower solve, upper solve
 template <class R>
@@ -497,7 +466,7 @@ void lu_solve_in_place_cx(cudaStream_t st, View<const R> L, View<const R> U, boo
   const i64 n = L.nrows;
   FB_ASSERT(L.ncols == n && U.nrows == n && U.ncols == n && rhs.nrows == n, "LU solve shape mismatch");
   if (n == 0 || rhs.ncols == 0) return;
-  permute_rows_cx<R>(st, rhs, perm_fwd);
+  permute_rows_in_place(st, as_pairs(rhs), perm_fwd);
   solve_lower_triangular_in_place_cx(st, L, true, conj, rhs);
   solve_upper_triangular_in_place_cx(st, U, false, conj, rhs);
 }
@@ -510,7 +479,7 @@ void lu_solve_transpose_in_place_cx(cudaStream_t st, View<const R> L, View<const
   if (n == 0 || rhs.ncols == 0) return;
   solve_lower_triangular_in_place_cx(st, U.t(), false, conj, rhs);
   solve_upper_triangular_in_place_cx(st, L.t(), true, conj, rhs);
-  permute_rows_cx<R>(st, rhs, perm_bwd);
+  permute_rows_in_place(st, as_pairs(rhs), perm_bwd);
 }
 
 // ---- Householder QR without pivoting for complex T (qr/no_pivoting/factor.rs:11-301; householder.rs:59-107, 132-272, 370-620,

@@ -1,8 +1,12 @@
-// extern "C" boundary: the symbols declared in include/faer_b200.h (second translation unit: ffi_types.cu, the entry points whose
-// drivers are the flat-map files; helpers shared by both: ffi_common.cuh).
-// Each entry point mirrors the faer-ffi function of the same name (faer-ffi/src/lib.rs, cited per function in the
-// header): same argument order and meaning, by-value PODs, synchronous on return, abort() on precondition
-// violations. Host buffers are staged; device buffers are used in place.
+// extern "C" boundary: the symbols declared in include/faer_b200.h. Each entry point mirrors the faer-ffi function of the same name
+// (faer-ffi/src/lib.rs, cited per function in the header): same argument order and meaning, by-value PODs, synchronous on return,
+// abort() on precondition violations. Host buffers are staged; device buffers are used in place.
+//
+// This unit holds the families whose drivers are the tensor-core files (matmul, triangular solves, LLT, LU, QR and the Householder
+// sequences, written once over the scalar kind <R, CX> with R the real type and CX "complex"), the f64 drivers of their own (LDLT,
+// reconstruct / inverse, svd / self_adjoint_evd for real T), the extensions and the global state. ffi_types.cu holds the entry
+// points of the flat-map drivers and every default-params / scratch query that is not QR's, LLT's or LU's: that unit also builds
+// for the host (tools/emul), this one does not. Helpers shared by both: ffi_common.cuh.
 #include "../../include/faer_b200.h"
 #include "ffi_common.cuh"
 #include "gemm_f32.cuh"
@@ -12,6 +16,7 @@
 #include <atomic>
 #include <cstring>
 #include <memory>
+#include <type_traits>
 #include <vector>
 
 using namespace fb;
@@ -21,171 +26,55 @@ namespace {
 std::atomic<int> g_par_tag{FaerV0_24_ParTag_Rayon};
 std::atomic<size_t> g_par_threads{0};
 
-inline size_t scalar_elem_f64() { return sizeof(double); }
+// ---- the drivers under the families: real T through the f64 / f32 overloads of tensor_ops.cuh and real_llt; complex T through the
+// cplx_* overloads (cplx.cu, gemm_c64.cu, gemm_c32.cu; views in complex-unit strides on an R* base, as the complex GEMMs take them) ----
+inline LltResult real_llt(cudaStream_t st, View<double> a, double delta, double eps, LltParams p) { return llt_cholesky_in_place_f64(st, a, delta, eps, p); }
+inline LltResult real_llt(cudaStream_t st, View<float> a, float delta, float eps, LltParams p) { return llt_cholesky_in_place_f32(st, a, delta, eps, p); }
+inline void cplx_gemm(cudaStream_t st, View<double> c, int cs, int acc, View<const double> a, int as, bool ca, View<const double> b, int bs, bool cb, double re, double im) { gemm_c64(st, c, cs, acc, a, as, ca, b, bs, cb, re, im); }
+inline void cplx_gemm(cudaStream_t st, View<float> c, int cs, int acc, View<const float> a, int as, bool ca, View<const float> b, int bs, bool cb, float re, float im) { gemm_c32(st, c, cs, acc, a, as, ca, b, bs, cb, re, im); }
+inline void cplx_solve_lower(cudaStream_t st, View<const double> t, bool unit, bool conj, View<double> r) { solve_lower_triangular_in_place_c64(st, t, unit, conj, r); }
+inline void cplx_solve_lower(cudaStream_t st, View<const float> t, bool unit, bool conj, View<float> r) { solve_lower_triangular_in_place_c32(st, t, unit, conj, r); }
+inline void cplx_solve_upper(cudaStream_t st, View<const double> t, bool unit, bool conj, View<double> r) { solve_upper_triangular_in_place_c64(st, t, unit, conj, r); }
+inline void cplx_solve_upper(cudaStream_t st, View<const float> t, bool unit, bool conj, View<float> r) { solve_upper_triangular_in_place_c32(st, t, unit, conj, r); }
+inline LltResult cplx_llt(cudaStream_t st, View<double> a, double delta, double eps) { return llt_cholesky_in_place_c64(st, a, delta, eps); }
+inline LltResult cplx_llt(cudaStream_t st, View<float> a, float delta, float eps) { return llt_cholesky_in_place_c32(st, a, delta, eps); }
+inline void cplx_llt_solve(cudaStream_t st, View<const double> l, bool conj, View<double> r) { llt_solve_in_place_c64(st, l, conj, r); }
+inline void cplx_llt_solve(cudaStream_t st, View<const float> l, bool conj, View<float> r) { llt_solve_in_place_c32(st, l, conj, r); }
+inline size_t cplx_lu(cudaStream_t st, View<double> a, long long* pf, long long* pb) { return lu_partial_piv_in_place_c64(st, a, pf, pb); }
+inline size_t cplx_lu(cudaStream_t st, View<float> a, long long* pf, long long* pb) { return lu_partial_piv_in_place_c32(st, a, pf, pb); }
+inline void cplx_lu_solve(cudaStream_t st, View<const double> l, View<const double> u, bool conj, const long long* p, View<double> r) { lu_solve_in_place_c64(st, l, u, conj, p, r); }
+inline void cplx_lu_solve(cudaStream_t st, View<const float> l, View<const float> u, bool conj, const long long* p, View<float> r) { lu_solve_in_place_c32(st, l, u, conj, p, r); }
+inline void cplx_lu_solve_t(cudaStream_t st, View<const double> l, View<const double> u, bool conj, const long long* p, View<double> r) { lu_solve_transpose_in_place_c64(st, l, u, conj, p, r); }
+inline void cplx_lu_solve_t(cudaStream_t st, View<const float> l, View<const float> u, bool conj, const long long* p, View<float> r) { lu_solve_transpose_in_place_c32(st, l, u, conj, p, r); }
+inline i64 cplx_qr(cudaStream_t st, View<double> a, View<double> q, i64 thr) { return qr_in_place_c64(st, a, q, thr); }
+inline i64 cplx_qr(cudaStream_t st, View<float> a, View<float> q, i64 thr) { return qr_in_place_c32(st, a, q, thr); }
+inline void cplx_hh_seq(cudaStream_t st, View<const double> b, View<const double> f, bool conj, View<double> r, bool tr) { apply_householder_sequence_left_c64(st, b, f, conj, r, tr); }
+inline void cplx_hh_seq(cudaStream_t st, View<const float> b, View<const float> f, bool conj, View<float> r, bool tr) { apply_householder_sequence_left_c32(st, b, f, conj, r, tr); }
 
-struct Mat {
-  StagedMat s;
-  Mat(FaerV0_24_MatRef m, cudaStream_t st)
-      : s(m.ptr, (i64)m.nrows, (i64)m.ncols, (i64)m.row_stride, (i64)m.col_stride, sizeof(double), true, false, st) {}
-  Mat(FaerV0_24_MatMut m, bool copy_in, cudaStream_t st)
-      : s(m.ptr, (i64)m.nrows, (i64)m.ncols, (i64)m.row_stride, (i64)m.col_stride, sizeof(double), copy_in, true, st) {}
-};
+// conj?(T) X = rhs with T lower or upper triangular; conj is a no-op for real T
+template <bool CX, class R>
+void tri_solve(cudaStream_t st, bool lower, View<const R> t, bool unit, bool conj, View<R> r) {
+  if constexpr (CX) {
+    if (lower) cplx_solve_lower(st, t, unit, conj, r);
+    else cplx_solve_upper(st, t, unit, conj, r);
+  } else {
+    if (lower) solve_lower(st, t, unit, r);
+    else solve_upper(st, t, unit, r);
+  }
+}
+// rhs <- op(Q) rhs (transpose = false) or op(Q)^H rhs (transpose = true) for the block-Householder sequence; conj is a no-op for real T
+template <bool CX, class R>
+void hh_seq(cudaStream_t st, View<const R> basis, View<const R> factor, bool conj, View<R> r, bool transpose) {
+  if constexpr (CX) cplx_hh_seq(st, basis, factor, conj, r, transpose);
+  else if (transpose) apply_block_householder_sequence_transpose_on_the_left<R>(st, basis, factor, r);
+  else apply_block_householder_sequence_on_the_left<R>(st, basis, factor, r);
+}
+// the leading m x n block of a view: no offset, so the same for real and complex-unit views
+template <class V>
+V leading(V v, i64 m, i64 n) { return V{v.ptr, m, n, v.rs, v.cs}; }
+inline FaerV0_24_MatMut transposed(FaerV0_24_MatMut m) { return FaerV0_24_MatMut{m.ptr, m.ncols, m.nrows, m.col_stride, m.row_stride}; }
 
-template <class S>
-void solve_tri(FaerV0_24_MatRef T, FaerV0_24_MatMut rhs, bool lower, bool unit) {
-  FB_ENTRY();
-  cudaStream_t st = current_stream();
-  FB_ASSERT(T.nrows == T.ncols && rhs.nrows == T.ncols, "triangular solve shape mismatch");
-  StagedMat t(T.ptr, (i64)T.nrows, (i64)T.ncols, (i64)T.row_stride, (i64)T.col_stride, sizeof(S), true, false, st);
-  StagedMat r(rhs.ptr, (i64)rhs.nrows, (i64)rhs.ncols, (i64)rhs.row_stride, (i64)rhs.col_stride, sizeof(S), true, true, st);
-  if (lower) solve_lower(st, t.view<const S>(), unit, r.view<S>());  // tensor_ops.cuh: f64 / f32 spellings of trsm.cu
-  else solve_upper(st, t.view<const S>(), unit, r.view<S>());
-  finish_all(st, {&t, &r});
-}
-
-// ---- Householder QR (no pivoting) + block-Householder sequence application, f64 and f32 ----
-template <class T>
-FaerV0_24_QrStatus qr_entry(FaerV0_24_MatMut A, FaerV0_24_MatMut Q) {
-  FB_ENTRY();
-  cudaStream_t st = current_stream();
-  const size_t size = A.nrows < A.ncols ? A.nrows : A.ncols;
-  FB_ASSERT(Q.nrows > 0 && Q.ncols == size, "Q_coeff must be block_size x min(nrows, ncols)");
-  StagedMat a(A.ptr, (i64)A.nrows, (i64)A.ncols, (i64)A.row_stride, (i64)A.col_stride, sizeof(T), true, true, st);
-  StagedMat q(Q.ptr, (i64)Q.nrows, (i64)Q.ncols, (i64)Q.row_stride, (i64)Q.col_stride, sizeof(T), true, true, st);
-  // the reference leaves the strict lower part of each T block untouched and zero-fills nothing for full rank
-  const i64 rank = qr_in_place<T>(st, a.view<T>(), q.view<T>());
-  finish_all(st, {&a, &q});
-  FaerV0_24_QrStatus out;
-  memset(&out, 0, sizeof(out));
-  if (rank < 0) {
-    out.tag = FaerV0_24_QrStatus_Unknown;
-  } else {
-    out.tag = FaerV0_24_QrStatus_Ok;
-    out.ok.rank = (size_t)rank;
-  }
-  return out;
-}
-inline FaerV0_24_MatMut transposed(FaerV0_24_MatMut m) {
-  return FaerV0_24_MatMut{m.ptr, m.ncols, m.nrows, m.col_stride, m.row_stride};
-}
-template <class T>
-void householder_seq_entry(FaerV0_24_MatRef basis, FaerV0_24_MatRef factor, FaerV0_24_MatMut rhs, bool transpose) {
-  FB_ENTRY();
-  cudaStream_t st = current_stream();
-  StagedMat b(basis.ptr, (i64)basis.nrows, (i64)basis.ncols, (i64)basis.row_stride, (i64)basis.col_stride, sizeof(T), true, false, st);
-  StagedMat f(factor.ptr, (i64)factor.nrows, (i64)factor.ncols, (i64)factor.row_stride, (i64)factor.col_stride, sizeof(T), true, false, st);
-  StagedMat r(rhs.ptr, (i64)rhs.nrows, (i64)rhs.ncols, (i64)rhs.row_stride, (i64)rhs.col_stride, sizeof(T), true, true, st);
-  if (transpose) apply_block_householder_sequence_transpose_on_the_left<T>(st, b.view<const T>(), f.view<const T>(), r.view<T>());
-  else apply_block_householder_sequence_on_the_left<T>(st, b.view<const T>(), f.view<const T>(), r.view<T>());
-  finish_all(st, {&b, &f, &r});
-}
-// ---- solves on the QR factors (qr/no_pivoting/solve.rs; SURVEY.md §8f rank 1) ----
-// mode 0: solve_lstsq_in_place_with_conj (solve.rs:38-76): rhs <- Q^H rhs, then R[..size, ..] x = rhs[..size, ..]
-// mode 1: solve_in_place_with_conj (solve.rs:96-119): the same on a square factorization
-// mode 2: solve_transpose_in_place_with_conj (solve.rs:140-176): rhs <- R^-T rhs (lower solve on the transposed view),
-//         then rhs <- conj(Q) rhs. Real scalar types only: the conj arguments are no-ops.
-template <class T>
-void qr_solve_entry(FaerV0_24_MatRef Qb, FaerV0_24_MatRef Qc, FaerV0_24_MatRef R, FaerV0_24_MatMut rhs, int mode) {
-  FB_ENTRY();
-  cudaStream_t st = current_stream();
-  const size_t m = Qb.nrows, n = Qb.ncols, size = m < n ? m : n;
-  FB_ASSERT(Qc.nrows > 0 && rhs.nrows == m && m >= n && Qc.ncols == size && R.nrows >= size && R.ncols == n,
-            "QR solve shape mismatch");
-  if (mode != 0) FB_ASSERT(m == n && R.nrows == n, "QR solve: the factorization must be square");
-  if (size == 0 || rhs.ncols == 0) return;
-  StagedMat b(Qb.ptr, (i64)m, (i64)n, (i64)Qb.row_stride, (i64)Qb.col_stride, sizeof(T), true, false, st);
-  StagedMat f(Qc.ptr, (i64)Qc.nrows, (i64)Qc.ncols, (i64)Qc.row_stride, (i64)Qc.col_stride, sizeof(T), true, false, st);
-  StagedMat r(rhs.ptr, (i64)rhs.nrows, (i64)rhs.ncols, (i64)rhs.row_stride, (i64)rhs.col_stride, sizeof(T), true, true, st);
-  // callers normally pass the packed QR matrix for both Q_basis and R (solve.rs:232-246): stage it once
-  const bool alias = R.ptr == Qb.ptr && R.row_stride == Qb.row_stride && R.col_stride == Qb.col_stride;
-  std::unique_ptr<StagedMat> rr;
-  if (!alias)
-    rr.reset(new StagedMat(R.ptr, (i64)size, (i64)n, (i64)R.row_stride, (i64)R.col_stride, sizeof(T), true, false, st));
-  View<const T> Rv = (alias ? b.view<const T>() : rr->view<const T>()).sub(0, 0, (i64)size, (i64)n);
-  View<T> x = r.view<T>();
-  if (mode == 2) {
-    solve_lower(st, Rv.t(), false, x);
-    apply_block_householder_sequence_on_the_left<T>(st, b.view<const T>(), f.view<const T>(), x);
-  } else {
-    apply_block_householder_sequence_transpose_on_the_left<T>(st, b.view<const T>(), f.view<const T>(), x);
-    solve_upper(st, Rv, false, x.sub(0, 0, (i64)size, x.ncols));
-  }
-  finish_all(st, {&b, &f, &r});
-  if (rr) rr->finish();
-}
-// ---- self-adjoint eigendecomposition (evd/mod.rs:270-418): eigenvalues by bisection when U is not wanted, divide and
-// conquer + Householder back-transform otherwise. Non-finite input -> EvdStatus::NoConvergence, as the reference ----
-template <class T>
-FaerV0_24_EvdStatus self_adjoint_evd_entry(FaerV0_24_MatRef A, FaerV0_24_MatMut U, FaerV0_24_VecMut S) {
-  FB_ENTRY();
-  cudaStream_t st = current_stream();
-  const size_t n = A.nrows;
-  FB_ASSERT(A.ncols == n && S.len == n && (n == 0 || S.stride >= 1), "self_adjoint_evd: square A, S of length n, positive stride");
-  const bool want_u = U.ncols != 0;
-  if (want_u) FB_ASSERT(U.nrows == n && U.ncols == n, "self_adjoint_evd: U must be n x n (or have no columns)");
-  FaerV0_24_EvdStatus out;
-  memset(&out, 0, sizeof(out));
-  out.tag = FaerV0_24_EvdStatus_Ok;
-  if (n == 0) return out;
-  StagedMat a(A.ptr, (i64)n, (i64)n, (i64)A.row_stride, (i64)A.col_stride, sizeof(T), true, false, st);
-  T* s_dev = (T*)ws_alloc(n * sizeof(T));
-  bool ok;
-  if (want_u) {
-    StagedMat u(U.ptr, (i64)n, (i64)n, (i64)U.row_stride, (i64)U.col_stride, sizeof(T), false, true, st);
-    ok = self_adjoint_evd_with_vectors<T>(st, a.view<const T>(), u.view<T>(), s_dev, 1);
-    if (ok) FB_CUDA_CHECK(cudaMemcpy2DAsync(S.ptr, (size_t)S.stride * sizeof(T), s_dev, sizeof(T), sizeof(T), n, cudaMemcpyDefault, st));
-    finish_all(st, {&a, &u});
-  } else {
-    ok = self_adjoint_eigenvalues<T>(st, a.view<const T>(), s_dev);
-    if (ok) FB_CUDA_CHECK(cudaMemcpy2DAsync(S.ptr, (size_t)S.stride * sizeof(T), s_dev, sizeof(T), sizeof(T), n, cudaMemcpyDefault, st));
-    finish_all(st, {&a});
-  }
-  ws_free(s_dev);
-  if (!ok) out.tag = FaerV0_24_EvdStatus_NoConvergence;
-  return out;
-}
-// ---- SVD (svd/mod.rs:530-672): U.ncols == 0 / V.ncols == 0 mean "do not compute" (faer-ffi/src/lib.rs:2354-2355) ----
-template <class T>
-FaerV0_24_SvdStatus svd_entry(FaerV0_24_MatRef A, FaerV0_24_MatMut U, FaerV0_24_VecMut S, FaerV0_24_MatMut V,
-                              double qr_ratio_threshold) {
-  FB_ENTRY();
-  cudaStream_t st = current_stream();
-  const size_t size = A.nrows < A.ncols ? A.nrows : A.ncols;
-  FB_ASSERT(S.len == size && (size == 0 || S.stride >= 1), "svd: S must have min(nrows, ncols) entries and a positive stride");
-  const bool want_u = U.ncols != 0, want_v = V.ncols != 0;
-  if (want_u) FB_ASSERT(U.nrows == A.nrows && (U.ncols == A.nrows || U.ncols == size), "svd: U must be nrows x {size, nrows}");
-  if (want_v) FB_ASSERT(V.nrows == A.ncols && (V.ncols == A.ncols || V.ncols == size), "svd: V must be ncols x {size, ncols}");
-  FaerV0_24_SvdStatus out;
-  memset(&out, 0, sizeof(out));
-  out.tag = FaerV0_24_SvdStatus_Ok;
-  const double ratio = qr_ratio_threshold > 0.0 ? qr_ratio_threshold : 11.0 / 6.0;
-  if (size == 0 && !want_u && !want_v) return out;
-  StagedMat a(A.ptr, (i64)A.nrows, (i64)A.ncols, (i64)A.row_stride, (i64)A.col_stride, sizeof(T), true, false, st);
-  T* s_dev = (T*)ws_alloc((size + 1) * sizeof(T));
-  bool ok;
-  if (want_u || want_v) {
-    StagedMat u(U.ptr, (i64)U.nrows, (i64)U.ncols, (i64)U.row_stride, (i64)U.col_stride, sizeof(T), false, true, st);
-    StagedMat v(V.ptr, (i64)V.nrows, (i64)V.ncols, (i64)V.row_stride, (i64)V.col_stride, sizeof(T), false, true, st);
-    View<T> uv = want_u ? u.view<T>() : View<T>{nullptr, 0, 0, 1, 1};
-    View<T> vv = want_v ? v.view<T>() : View<T>{nullptr, 0, 0, 1, 1};
-    ok = svd_with_vectors<T>(st, a.view<const T>(), uv, s_dev, 1, vv, ratio);
-    if (ok && size)
-      FB_CUDA_CHECK(cudaMemcpy2DAsync(S.ptr, (size_t)S.stride * sizeof(T), s_dev, sizeof(T), sizeof(T), size, cudaMemcpyDefault, st));
-    finish_all(st, {&a, &u, &v});
-  } else {
-    ok = singular_values<T>(st, a.view<const T>(), s_dev, ratio);
-    // strided scatter into the caller's vector (host or device)
-    if (ok) FB_CUDA_CHECK(cudaMemcpy2DAsync(S.ptr, (size_t)S.stride * sizeof(T), s_dev, sizeof(T), sizeof(T), size, cudaMemcpyDefault, st));
-    finish_all(st, {&a});
-  }
-  ws_free(s_dev);
-  if (!ok) out.tag = FaerV0_24_SvdStatus_NoConvergence;
-  return out;
-}
-}  // namespace
-
-// widening / narrowing copies and the f32 row gather of the f32 LU entry points (below)
-namespace {
+// widening / narrowing copies of the f32 LU factorization (below)
 template <class TD, class TS>
 __global__ void ffi_cast_kernel(TD* __restrict__ dst, i64 drs, i64 dcs, const TS* __restrict__ src, i64 srs, i64 scs, i64 m,
                                 i64 c0) {
@@ -203,443 +92,354 @@ void ffi_cast(cudaStream_t st, TD* dst, i64 drs, i64 dcs, const TS* src, i64 srs
   }
   FB_CUDA_CHECK(cudaGetLastError());
 }
-__global__ void ffi_gather_rows_f32_kernel(float* __restrict__ dst, const float* __restrict__ src, i64 rs, i64 cs, i64 nrows,
-                                           const long long* __restrict__ perm) {
-  const i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x;
-  const i64 c = blockIdx.y;
-  if (i < nrows) dst[c * nrows + i] = src[perm[i] * rs + c * cs];
+
+// ---- matmul (f64: DMMA, f32: 3xTF32 tensor-core kernel, c64 / c32: the complex GEMMs; `alpha` points to a T-typed scalar) ----
+template <class R, bool CX>
+void matmul_entry(FaerV0_24_MatMut C, int C_block, FaerV0_24_Accum accum, FaerV0_24_MatRef A, int A_block, FaerV0_24_MatRef B,
+                  int B_block, const FaerV0_24_Scalar* alpha, bool conj_a = false, bool conj_b = false) {
+  FB_ENTRY();
+  FB_ASSERT(C.nrows == A.nrows && C.ncols == B.ncols && A.ncols == B.nrows, "matmul shape mismatch");
+  cudaStream_t st = current_stream();
+  R a[2] = {0, 0};
+  read_scalar(alpha, a, CX ? 2 : 1);
+  const size_t es = elem_bytes<R, CX>();
+  const int add = accum == FaerV0_24_Accum_Add ? 1 : 0;
+  StagedMat c = stage(C, es, add || C_block != FaerV0_24_Block_Rectangular, st), l = stage(A, es, st), r = stage(B, es, st);
+  if constexpr (CX)
+    cplx_gemm(st, c.view<R>(), C_block, add, l.view<const R>(), A_block, conj_a, r.view<const R>(), B_block, conj_b, a[0], a[1]);
+  else
+    gemm(st, c.view<R>(), C_block, add, l.view<const R>(), A_block, r.view<const R>(), B_block, a[0]);
+  finish_all(st, {&c, &l, &r});
 }
-}  // namespace
 
-
-
-// ---- complex (c64 / c32) triangular solves, LLT and partial-pivoting LU: cplx.cu, templated over the real type R; the device
-// views are in complex-unit strides on an R* base, as the complex GEMMs take them ----
-inline void cplx_solve_lower(cudaStream_t st, View<const double> t, bool unit, bool conj, View<double> r) { solve_lower_triangular_in_place_c64(st, t, unit, conj, r); }
-inline void cplx_solve_lower(cudaStream_t st, View<const float> t, bool unit, bool conj, View<float> r) { solve_lower_triangular_in_place_c32(st, t, unit, conj, r); }
-inline void cplx_solve_upper(cudaStream_t st, View<const double> t, bool unit, bool conj, View<double> r) { solve_upper_triangular_in_place_c64(st, t, unit, conj, r); }
-inline void cplx_solve_upper(cudaStream_t st, View<const float> t, bool unit, bool conj, View<float> r) { solve_upper_triangular_in_place_c32(st, t, unit, conj, r); }
-inline LltResult cplx_llt(cudaStream_t st, View<double> a, double delta, double eps) { return llt_cholesky_in_place_c64(st, a, delta, eps); }
-inline LltResult cplx_llt(cudaStream_t st, View<float> a, float delta, float eps) { return llt_cholesky_in_place_c32(st, a, delta, eps); }
-inline void cplx_llt_solve(cudaStream_t st, View<const double> l, bool conj, View<double> r) { llt_solve_in_place_c64(st, l, conj, r); }
-inline void cplx_llt_solve(cudaStream_t st, View<const float> l, bool conj, View<float> r) { llt_solve_in_place_c32(st, l, conj, r); }
-inline size_t cplx_lu(cudaStream_t st, View<double> a, long long* pf, long long* pb) { return lu_partial_piv_in_place_c64(st, a, pf, pb); }
-inline size_t cplx_lu(cudaStream_t st, View<float> a, long long* pf, long long* pb) { return lu_partial_piv_in_place_c32(st, a, pf, pb); }
-inline void cplx_lu_solve(cudaStream_t st, View<const double> l, View<const double> u, bool conj, const long long* p, View<double> r) { lu_solve_in_place_c64(st, l, u, conj, p, r); }
-inline void cplx_lu_solve(cudaStream_t st, View<const float> l, View<const float> u, bool conj, const long long* p, View<float> r) { lu_solve_in_place_c32(st, l, u, conj, p, r); }
-inline void cplx_lu_solve_t(cudaStream_t st, View<const double> l, View<const double> u, bool conj, const long long* p, View<double> r) { lu_solve_transpose_in_place_c64(st, l, u, conj, p, r); }
-inline void cplx_lu_solve_t(cudaStream_t st, View<const float> l, View<const float> u, bool conj, const long long* p, View<float> r) { lu_solve_transpose_in_place_c32(st, l, u, conj, p, r); }
-
-template <class R>
-void solve_tri_cplx(FaerV0_24_MatRef T, FaerV0_24_Conj conj, FaerV0_24_MatMut rhs, bool lower, bool unit) {
+// ---- triangular solves (trsm.cu for real T, cplx.cu for complex T) ----
+template <class R, bool CX>
+void solve_tri_entry(FaerV0_24_MatRef T, FaerV0_24_Conj conj, FaerV0_24_MatMut rhs, bool lower, bool unit) {
   FB_ENTRY();
   FB_ASSERT(T.nrows == T.ncols && rhs.nrows == T.nrows, "triangular solve shape mismatch");
   cudaStream_t st = current_stream();
-  StagedMat t(T.ptr, (i64)T.nrows, (i64)T.ncols, (i64)T.row_stride, (i64)T.col_stride, 2 * sizeof(R), true, false, st);
-  StagedMat r(rhs.ptr, (i64)rhs.nrows, (i64)rhs.ncols, (i64)rhs.row_stride, (i64)rhs.col_stride, 2 * sizeof(R), true, true, st);
-  if (lower) cplx_solve_lower(st, t.view<const R>(), unit, conj == FaerV0_24_Conj_Yes, r.view<R>());
-  else cplx_solve_upper(st, t.view<const R>(), unit, conj == FaerV0_24_Conj_Yes, r.view<R>());
+  const size_t es = elem_bytes<R, CX>();
+  StagedMat t = stage(T, es, st), r = stage(rhs, es, true, st);
+  tri_solve<CX>(st, lower, t.view<const R>(), unit, CX && conj == FaerV0_24_Conj_Yes, r.view<R>());
   finish_all(st, {&t, &r});
 }
-template <class R>
-FaerV0_24_LltStatus llt_factor_cplx(FaerV0_24_MatMut A, FaerV0_24_LltRegularization regularization) {
+
+// ---- LLT (llt.cu for real T, cplx.cu for complex T) ----
+template <class R, bool CX>
+FaerV0_24_LltStatus llt_factor_entry(FaerV0_24_MatMut A, FaerV0_24_LltRegularization regularization, FaerV0_24_LltParams params) {
   FB_ENTRY();
   FB_ASSERT(A.nrows == A.ncols, "LLT needs a square matrix");
   cudaStream_t st = current_stream();
-  R delta = 0, eps = 0;  // the regularisation parameters are T::Real
-  if (regularization.dynamic_regularization_delta) delta = read_real(regularization.dynamic_regularization_delta, R());
-  if (regularization.dynamic_regularization_epsilon) eps = read_real(regularization.dynamic_regularization_epsilon, R());
-  StagedMat a(A.ptr, (i64)A.nrows, (i64)A.ncols, (i64)A.row_stride, (i64)A.col_stride, 2 * sizeof(R), true, true, st);
-  const LltResult r = cplx_llt(st, a.view<R>(), delta, eps);
-  finish_all(st, {&a});
-  FaerV0_24_LltStatus out;
-  memset(&out, 0, sizeof(out));
-  if (r.ok) {
-    out.tag = FaerV0_24_LltStatus_Ok;
-    out.ok.dynamic_regularization_count = r.dynamic_regularization_count;
-  } else {
-    out.tag = FaerV0_24_LltStatus_NonPositivePivot;
-    out.non_positive_pivot.index = r.non_positive_pivot_index;
+  R delta, eps;  // the regularisation parameters are T::Real
+  read_regularization(regularization, delta, eps);
+  if constexpr (std::is_same<R, double>::value && !CX) {
+    // f64 host matrix, column-major and large: upload / factor / download pipelined block column by block column (dist.cu)
+    if (A.nrows > 0 && !is_device_pointer(A.ptr) && A.row_stride == 1 && A.col_stride >= (ptrdiff_t)A.nrows &&
+        (i64)A.nrows >= lookahead_min_n()) {
+      FB_CUDA_CHECK(cudaStreamSynchronize(st));
+      const i64 nb = lookahead_block() ? lookahead_block() : 256;
+      return llt_status(llt_host_pipelined_f64((double*)A.ptr, (i64)A.col_stride, (i64)A.nrows, nb, delta, eps));
+    }
   }
-  return out;
+  StagedMat a = stage(A, elem_bytes<R, CX>(), true, st);
+  LltResult r;
+  if constexpr (CX) r = cplx_llt(st, a.view<R>(), delta, eps);  // the complex driver has no tuning parameters
+  else r = real_llt(st, a.view<R>(), delta, eps, LltParams{params.recursion_threshold, params.block_size});
+  finish_all(st, {&a});
+  return llt_status(r);
 }
-template <class R>
-void llt_solve_cplx(FaerV0_24_MatRef L, FaerV0_24_Conj A_conj, FaerV0_24_MatMut rhs) {
+template <class R, bool CX>
+void llt_solve_entry(FaerV0_24_MatRef L, FaerV0_24_Conj A_conj, FaerV0_24_MatMut rhs) {
   FB_ENTRY();
   FB_ASSERT(L.nrows == L.ncols && rhs.nrows == L.nrows, "LLT solve shape mismatch");
   cudaStream_t st = current_stream();
-  StagedMat l(L.ptr, (i64)L.nrows, (i64)L.ncols, (i64)L.row_stride, (i64)L.col_stride, 2 * sizeof(R), true, false, st);
-  StagedMat r(rhs.ptr, (i64)rhs.nrows, (i64)rhs.ncols, (i64)rhs.row_stride, (i64)rhs.col_stride, 2 * sizeof(R), true, true, st);
-  cplx_llt_solve(st, l.view<const R>(), A_conj == FaerV0_24_Conj_Yes, r.view<R>());
+  const size_t es = elem_bytes<R, CX>();
+  StagedMat l = stage(L, es, st), r = stage(rhs, es, true, st);
+  if constexpr (CX) cplx_llt_solve(st, l.view<const R>(), A_conj == FaerV0_24_Conj_Yes, r.view<R>());
+  else llt_solve_in_place(st, l.view<const R>(), r.view<R>());
   finish_all(st, {&l, &r});
 }
-template <class R>
-FaerV0_24_PartialPivLuStatus lu_entry_cplx(FaerV0_24_MatMut A, FaerV0_24_SliceMut perm_fwd, FaerV0_24_SliceMut perm_bwd, int idx_bytes) {
+
+// ---- partial-pivoting LU (lu_f64.cu for f64 and f32, cplx.cu for complex T) ----
+template <class R, bool CX>
+FaerV0_24_PartialPivLuStatus lu_factor_entry(FaerV0_24_MatMut A, FaerV0_24_SliceMut perm_fwd, FaerV0_24_SliceMut perm_bwd,
+                                             FaerV0_24_PartialPivLuParams params, int idx_bytes) {
   FB_ENTRY();
   cudaStream_t st = current_stream();
+  // faer.hpp fills SliceMut.len with bytes (ffi_common.cuh): the permutation length is A.nrows
   FB_ASSERT(A.nrows == 0 || (perm_fwd.ptr != nullptr && perm_bwd.ptr != nullptr), "null permutation slice");
-  StagedMat a(A.ptr, (i64)A.nrows, (i64)A.ncols, (i64)A.row_stride, (i64)A.col_stride, 2 * sizeof(R), true, true, st);
-  std::vector<long long> pf(A.nrows), pb(A.nrows);
-  const size_t cnt = cplx_lu(st, a.view<R>(), pf.data(), pb.data());
+  StagedMat a = stage(A, elem_bytes<R, CX>(), true, st);
+  const PartialPivLuParams p{params.recursion_threshold, params.block_size, params.par_threshold};
+  size_t cnt;
+  std::vector<long long> pf, pb;
+  double* W = nullptr;
+  if constexpr (CX) {
+    // the complex driver returns host permutations and has no tuning parameters
+    pf.resize(A.nrows);
+    pb.resize(A.nrows);
+    cnt = cplx_lu(st, a.view<R>(), pf.data(), pb.data());
+  } else if constexpr (std::is_same<R, float>::value) {
+    // f32 is computed in f64: the matrix is widened on the device, factored by the f64 drivers (fused sub-panel kernel, TMA-fed
+    // GEMM, SM partition) and rounded back. The factors carry one f32 rounding instead of an f32 elimination's accumulated ones,
+    // and the pivot search sees f64 values (a pivot can differ from an all-f32 elimination's where two candidates agree to f32
+    // precision; either choice is a valid partial pivot). The solves run on the native f32 triangular solves.
+    const i64 m = (i64)A.nrows, n = (i64)A.ncols;
+    VF av = a.view<float>();
+    const i64 ld = std::max<i64>(1, (m + 1) & ~(i64)1);
+    W = (double*)ws_alloc((size_t)ld * (size_t)std::max<i64>(n, 1) * 8);
+    ffi_cast<double, float>(st, W, 1, ld, av.ptr, av.rs, av.cs, m, n);
+    cnt = lu_partial_piv_in_place_f64(st, VD{W, m, n, 1, ld}, perm_fwd.ptr, perm_bwd.ptr, idx_bytes, p);
+    ffi_cast<float, double>(st, av.ptr, av.rs, av.cs, W, 1, ld, m, n);
+  } else {
+    cnt = lu_partial_piv_in_place_f64(st, a.view<double>(), perm_fwd.ptr, perm_bwd.ptr, idx_bytes, p);
+  }
   finish_all(st, {&a});
-  write_perm(perm_fwd.ptr, pf, idx_bytes);
-  write_perm(perm_bwd.ptr, pb, idx_bytes);
-  FaerV0_24_PartialPivLuStatus out;
-  memset(&out, 0, sizeof(out));
-  out.tag = FaerV0_24_PartialPivLuStatus_Ok;
-  out.ok.transposition_count = cnt;
-  return out;
+  if (W) ws_free(W);
+  if constexpr (CX) {
+    write_perm(perm_fwd.ptr, pf, idx_bytes);
+    write_perm(perm_bwd.ptr, pb, idx_bytes);
+  }
+  return lu_status(cnt);
 }
-template <class R>
-void lu_solve_entry_cplx(FaerV0_24_MatRef L, FaerV0_24_MatRef U, FaerV0_24_Conj conj, FaerV0_24_SliceRef perm_slice, FaerV0_24_MatMut rhs,
-                         int idx_bytes, bool transpose = false) {
+// transpose = false: perm is perm_fwd (solve.rs:21-54); transpose = true: perm is perm_bwd (solve.rs:55-86)
+template <class R, bool CX>
+void lu_solve_entry(FaerV0_24_MatRef L, FaerV0_24_MatRef U, FaerV0_24_Conj conj, FaerV0_24_SliceRef perm_slice, FaerV0_24_MatMut rhs,
+                    int idx_bytes, bool transpose) {
   FB_ENTRY();
   cudaStream_t st = current_stream();
   const size_t n = L.nrows;
   FB_ASSERT(L.ncols == n && U.nrows == n && U.ncols == n && rhs.nrows == n, "LU solve shape mismatch");
-  std::vector<long long> perm = read_perm(perm_slice.ptr, n, idx_bytes);
-  for (size_t i = 0; i < n; ++i) FB_ASSERT(perm[i] >= 0 && (size_t)perm[i] < n, "invalid permutation entry");
-  StagedMat l(L.ptr, (i64)L.nrows, (i64)L.ncols, (i64)L.row_stride, (i64)L.col_stride, 2 * sizeof(R), true, false, st);
-  StagedMat u(U.ptr, (i64)U.nrows, (i64)U.ncols, (i64)U.row_stride, (i64)U.col_stride, 2 * sizeof(R), true, false, st);
-  StagedMat r(rhs.ptr, (i64)rhs.nrows, (i64)rhs.ncols, (i64)rhs.row_stride, (i64)rhs.col_stride, 2 * sizeof(R), true, true, st);
-  // transpose = false: perm is perm_fwd (solve.rs:21-54); transpose = true: perm is perm_bwd (solve.rs:55-86)
-  if (transpose) cplx_lu_solve_t(st, l.view<const R>(), u.view<const R>(), conj == FaerV0_24_Conj_Yes, perm.data(), r.view<R>());
-  else cplx_lu_solve(st, l.view<const R>(), u.view<const R>(), conj == FaerV0_24_Conj_Yes, perm.data(), r.view<R>());
+  const std::vector<long long> perm = read_perm_checked(perm_slice, n, idx_bytes);
+  const size_t es = elem_bytes<R, CX>();
+  StagedMat l = stage(L, es, st), u = stage(U, es, st), r = stage(rhs, es, true, st);
+  if constexpr (CX) {
+    const bool cj = conj == FaerV0_24_Conj_Yes;
+    if (transpose) cplx_lu_solve_t(st, l.view<const R>(), u.view<const R>(), cj, perm.data(), r.view<R>());
+    else cplx_lu_solve(st, l.view<const R>(), u.view<const R>(), cj, perm.data(), r.view<R>());
+  } else {
+    if (transpose) lu_solve_transpose_in_place(st, l.view<const R>(), u.view<const R>(), perm.data(), r.view<R>());
+    else lu_solve_in_place(st, l.view<const R>(), u.view<const R>(), perm.data(), r.view<R>());
+  }
   finish_all(st, {&l, &u, &r});
 }
 
-
-// complex Householder QR / block-Householder sequences / QR solves (cplx.cu)
-inline i64 cplx_qr(cudaStream_t st, View<double> a, View<double> q, i64 thr) { return qr_in_place_c64(st, a, q, thr); }
-inline i64 cplx_qr(cudaStream_t st, View<float> a, View<float> q, i64 thr) { return qr_in_place_c32(st, a, q, thr); }
-inline void cplx_hh_seq(cudaStream_t st, View<const double> b, View<const double> f, bool conj, View<double> r, bool tr) { apply_householder_sequence_left_c64(st, b, f, conj, r, tr); }
-inline void cplx_hh_seq(cudaStream_t st, View<const float> b, View<const float> f, bool conj, View<float> r, bool tr) { apply_householder_sequence_left_c32(st, b, f, conj, r, tr); }
-template <class V>
-inline V cplx_sub(V v, i64 i, i64 j, i64 m, i64 n) { return V{v.ptr + 2 * (i * v.rs + j * v.cs), m, n, v.rs, v.cs}; }
-
-template <class R>
-FaerV0_24_QrStatus qr_entry_cplx(FaerV0_24_MatMut A, FaerV0_24_MatMut Q, FaerV0_24_QrParams params) {
+// ---- Householder QR (no pivoting), block-Householder sequences and the solves on the QR factors (qr.cu / householder.cu for real
+// T, cplx.cu for complex T) ----
+template <class R, bool CX>
+FaerV0_24_QrStatus qr_factor_entry(FaerV0_24_MatMut A, FaerV0_24_MatMut Q, FaerV0_24_QrParams params) {
   FB_ENTRY();
   cudaStream_t st = current_stream();
   const size_t size = A.nrows < A.ncols ? A.nrows : A.ncols;
   FB_ASSERT(Q.nrows > 0 && Q.ncols == size, "Q_coeff must be block_size x min(nrows, ncols)");
-  StagedMat a(A.ptr, (i64)A.nrows, (i64)A.ncols, (i64)A.row_stride, (i64)A.col_stride, 2 * sizeof(R), true, true, st);
-  StagedMat q(Q.ptr, (i64)Q.nrows, (i64)Q.ncols, (i64)Q.row_stride, (i64)Q.col_stride, 2 * sizeof(R), true, true, st);
-  const i64 rank = cplx_qr(st, a.view<R>(), q.view<R>(), (i64)params.blocking_threshold);
+  const size_t es = elem_bytes<R, CX>();
+  StagedMat a = stage(A, es, true, st), q = stage(Q, es, true, st);
+  // the reference leaves the strict lower part of each T block untouched and zero-fills nothing for full rank
+  i64 rank;
+  if constexpr (CX) rank = cplx_qr(st, a.view<R>(), q.view<R>(), (i64)params.blocking_threshold);
+  else rank = qr_in_place<R>(st, a.view<R>(), q.view<R>());  // the real driver picks its own blocking
   finish_all(st, {&a, &q});
-  FaerV0_24_QrStatus out;
-  memset(&out, 0, sizeof(out));
-  out.tag = FaerV0_24_QrStatus_Ok;
-  out.ok.rank = (size_t)rank;
-  return out;
+  return qr_status(CX || rank >= 0, (size_t)rank);  // only the real driver reports an unknown rank (< 0)
 }
-template <class R>
-void householder_seq_entry_cplx(FaerV0_24_MatRef basis, FaerV0_24_MatRef factor, FaerV0_24_Conj conj, FaerV0_24_MatMut rhs, bool transpose) {
+template <class R, bool CX>
+void householder_seq_entry(FaerV0_24_MatRef basis, FaerV0_24_MatRef factor, FaerV0_24_Conj conj, FaerV0_24_MatMut rhs, bool transpose) {
   FB_ENTRY();
   cudaStream_t st = current_stream();
-  StagedMat b(basis.ptr, (i64)basis.nrows, (i64)basis.ncols, (i64)basis.row_stride, (i64)basis.col_stride, 2 * sizeof(R), true, false, st);
-  StagedMat f(factor.ptr, (i64)factor.nrows, (i64)factor.ncols, (i64)factor.row_stride, (i64)factor.col_stride, 2 * sizeof(R), true, false, st);
-  StagedMat r(rhs.ptr, (i64)rhs.nrows, (i64)rhs.ncols, (i64)rhs.row_stride, (i64)rhs.col_stride, 2 * sizeof(R), true, true, st);
-  cplx_hh_seq(st, b.view<const R>(), f.view<const R>(), conj == FaerV0_24_Conj_Yes, r.view<R>(), transpose);
+  const size_t es = elem_bytes<R, CX>();
+  StagedMat b = stage(basis, es, st), f = stage(factor, es, st), r = stage(rhs, es, true, st);
+  hh_seq<CX>(st, b.view<const R>(), f.view<const R>(), CX && conj == FaerV0_24_Conj_Yes, r.view<R>(), transpose);
   finish_all(st, {&b, &f, &r});
 }
-// qr/no_pivoting/solve.rs:38-176 for complex T. mode 0: least squares (m >= n), 1: square solve, 2: transpose solve
-template <class R>
-void qr_solve_entry_cplx(FaerV0_24_MatRef Qb, FaerV0_24_MatRef Qc, FaerV0_24_MatRef Rm, FaerV0_24_Conj A_conj, FaerV0_24_MatMut rhs, int mode) {
+// qr/no_pivoting/solve.rs; SURVEY.md §8f rank 1:
+// mode 0: solve_lstsq_in_place_with_conj (solve.rs:38-76): rhs <- op(Q)^H rhs, then op(R)[..size, ..] x = rhs[..size, ..]
+// mode 1: solve_in_place_with_conj (solve.rs:96-119): the same on a square factorization
+// mode 2: solve_transpose_in_place_with_conj (solve.rs:140-176): op(R)^T y = rhs (lower solve on the transposed view), then
+//         rhs <- the forward sequence with conj composed with Yes
+template <class R, bool CX>
+void qr_solve_entry(FaerV0_24_MatRef Qb, FaerV0_24_MatRef Qc, FaerV0_24_MatRef Rm, FaerV0_24_Conj A_conj, FaerV0_24_MatMut rhs, int mode) {
   FB_ENTRY();
   cudaStream_t st = current_stream();
   const size_t m = Qb.nrows, n = Qb.ncols, size = m < n ? m : n;
   FB_ASSERT(Qc.nrows > 0 && rhs.nrows == m && m >= n && Qc.ncols == size && Rm.nrows >= size && Rm.ncols == n, "QR solve shape mismatch");
   if (mode != 0) FB_ASSERT(m == n && Rm.nrows == n, "QR solve: the factorization must be square");
   if (size == 0 || rhs.ncols == 0) return;
-  const bool conj = A_conj == FaerV0_24_Conj_Yes;
-  StagedMat b(Qb.ptr, (i64)m, (i64)n, (i64)Qb.row_stride, (i64)Qb.col_stride, 2 * sizeof(R), true, false, st);
-  StagedMat f(Qc.ptr, (i64)Qc.nrows, (i64)Qc.ncols, (i64)Qc.row_stride, (i64)Qc.col_stride, 2 * sizeof(R), true, false, st);
-  StagedMat r(rhs.ptr, (i64)rhs.nrows, (i64)rhs.ncols, (i64)rhs.row_stride, (i64)rhs.col_stride, 2 * sizeof(R), true, true, st);
+  const bool conj = CX && A_conj == FaerV0_24_Conj_Yes;
+  const size_t es = elem_bytes<R, CX>();
+  StagedMat b = stage(Qb, es, st), f = stage(Qc, es, st), r = stage(rhs, es, true, st);
+  // callers normally pass the packed QR matrix for both Q_basis and R (solve.rs:232-246): stage it once
   const bool alias = Rm.ptr == Qb.ptr && Rm.row_stride == Qb.row_stride && Rm.col_stride == Qb.col_stride;
   std::unique_ptr<StagedMat> rr;
-  if (!alias) rr.reset(new StagedMat(Rm.ptr, (i64)size, (i64)n, (i64)Rm.row_stride, (i64)Rm.col_stride, 2 * sizeof(R), true, false, st));
-  View<const R> Rv = cplx_sub(alias ? b.view<const R>() : rr->view<const R>(), 0, 0, (i64)size, (i64)n);
+  if (!alias) rr.reset(new StagedMat(Rm.ptr, (i64)size, (i64)n, (i64)Rm.row_stride, (i64)Rm.col_stride, es, true, false, st));
+  View<const R> Rv = leading(alias ? b.view<const R>() : rr->view<const R>(), (i64)size, (i64)n);
   View<R> x = r.view<R>();
   if (mode == 2) {
-    cplx_solve_lower(st, Rv.t(), false, conj, x);               // op(R)^T y = rhs
-    cplx_hh_seq(st, b.view<const R>(), f.view<const R>(), !conj, x, false);  // the forward sequence with conj composed with Yes
+    tri_solve<CX>(st, true, Rv.t(), false, conj, x);
+    hh_seq<CX>(st, b.view<const R>(), f.view<const R>(), !conj, x, false);
   } else {
-    cplx_hh_seq(st, b.view<const R>(), f.view<const R>(), !conj, x, true);   // op(Q)^H rhs
-    cplx_solve_upper(st, Rv, false, conj, cplx_sub(x, 0, 0, (i64)size, x.ncols));
+    hh_seq<CX>(st, b.view<const R>(), f.view<const R>(), !conj, x, true);
+    tri_solve<CX>(st, false, Rv, false, conj, leading(x, (i64)size, x.ncols));
   }
   finish_all(st, {&b, &f, &r});
   if (rr) rr->finish();
 }
 
+// ---- self-adjoint eigendecomposition for real T (evd/mod.rs:270-418): eigenvalues by bisection when U is not wanted, divide and
+// conquer + Householder back-transform otherwise. Non-finite input -> EvdStatus::NoConvergence, as the reference ----
+template <class T>
+FaerV0_24_EvdStatus self_adjoint_evd_entry(FaerV0_24_MatRef A, FaerV0_24_MatMut U, FaerV0_24_VecMut S) {
+  FB_ENTRY();
+  cudaStream_t st = current_stream();
+  const size_t n = A.nrows;
+  FB_ASSERT(A.ncols == n && S.len == n && (n == 0 || S.stride >= 1), "self_adjoint_evd: square A, S of length n, positive stride");
+  const bool want_u = U.ncols != 0;
+  if (want_u) FB_ASSERT(U.nrows == n && U.ncols == n, "self_adjoint_evd: U must be n x n (or have no columns)");
+  if (n == 0) return evd_status(true);
+  StagedMat a = stage(A, sizeof(T), st);
+  T* s_dev = (T*)ws_alloc(n * sizeof(T));
+  bool ok;
+  if (want_u) {
+    StagedMat u = stage(U, sizeof(T), false, st);
+    ok = self_adjoint_evd_with_vectors<T>(st, a.view<const T>(), u.view<T>(), s_dev, 1);
+    if (ok) copy_out_vector(S, s_dev, n, sizeof(T), st);
+    finish_all(st, {&a, &u});
+  } else {
+    ok = self_adjoint_eigenvalues<T>(st, a.view<const T>(), s_dev);
+    if (ok) copy_out_vector(S, s_dev, n, sizeof(T), st);
+    finish_all(st, {&a});
+  }
+  ws_free(s_dev);
+  return evd_status(ok);
+}
+// ---- SVD for real T (svd/mod.rs:530-672): U.ncols == 0 / V.ncols == 0 mean "do not compute" (faer-ffi/src/lib.rs:2354-2355) ----
+template <class T>
+FaerV0_24_SvdStatus svd_entry(FaerV0_24_MatRef A, FaerV0_24_MatMut U, FaerV0_24_VecMut S, FaerV0_24_MatMut V,
+                              double qr_ratio_threshold) {
+  FB_ENTRY();
+  cudaStream_t st = current_stream();
+  const size_t size = A.nrows < A.ncols ? A.nrows : A.ncols;
+  FB_ASSERT(S.len == size && (size == 0 || S.stride >= 1), "svd: S must have min(nrows, ncols) entries and a positive stride");
+  const bool want_u = U.ncols != 0, want_v = V.ncols != 0;
+  if (want_u) FB_ASSERT(U.nrows == A.nrows && (U.ncols == A.nrows || U.ncols == size), "svd: U must be nrows x {size, nrows}");
+  if (want_v) FB_ASSERT(V.nrows == A.ncols && (V.ncols == A.ncols || V.ncols == size), "svd: V must be ncols x {size, ncols}");
+  const double ratio = qr_ratio_threshold > 0.0 ? qr_ratio_threshold : 11.0 / 6.0;
+  if (size == 0 && !want_u && !want_v) return svd_status(true);
+  StagedMat a = stage(A, sizeof(T), st);
+  T* s_dev = (T*)ws_alloc((size + 1) * sizeof(T));
+  bool ok;
+  if (want_u || want_v) {
+    StagedMat u = stage(U, sizeof(T), false, st), v = stage(V, sizeof(T), false, st);
+    View<T> uv = want_u ? u.view<T>() : View<T>{nullptr, 0, 0, 1, 1};
+    View<T> vv = want_v ? v.view<T>() : View<T>{nullptr, 0, 0, 1, 1};
+    ok = svd_with_vectors<T>(st, a.view<const T>(), uv, s_dev, 1, vv, ratio);
+    if (ok && size) copy_out_vector(S, s_dev, size, sizeof(T), st);
+    finish_all(st, {&a, &u, &v});
+  } else {
+    ok = singular_values<T>(st, a.view<const T>(), s_dev, ratio);
+    if (ok) copy_out_vector(S, s_dev, size, sizeof(T), st);
+    finish_all(st, {&a});
+  }
+  ws_free(s_dev);
+  return svd_status(ok);
+}
+
+// f64 reconstruct / inverse on the LU factors (reconstruct.cu)
+void lu_recon_entry(FaerV0_24_MatMut A, FaerV0_24_MatRef L, FaerV0_24_MatRef U, FaerV0_24_SliceRef perm, int idx_bytes, bool inverse) {
+  FB_ENTRY();
+  cudaStream_t st = current_stream();
+  const std::vector<long long> p = read_perm_checked(perm, L.nrows, idx_bytes);
+  StagedMat a = stage(A, sizeof(double), false, st), l = stage(L, sizeof(double), st), u = stage(U, sizeof(double), st);
+  if (inverse) lu_inverse_f64(st, a.view<double>(), l.view<const double>(), u.view<const double>(), p.data());
+  else lu_reconstruct_f64(st, a.view<double>(), l.view<const double>(), u.view<const double>(), p.data());
+  finish_all(st, {&a, &l, &u});
+}
+
+}  // namespace
+
 extern "C" {
 
-void libfaer_v0_23_matmul_f64(FaerV0_24_MatMut C, FaerV0_24_Accum accum, FaerV0_24_MatRef A, FaerV0_24_MatRef B,
-                              const FaerV0_24_Scalar* alpha, FaerV0_24_Par par) {
-  (void)par;
-  FB_ENTRY();
-  FB_ASSERT(C.nrows == A.nrows && C.ncols == B.ncols && A.ncols == B.nrows, "matmul shape mismatch");
-  cudaStream_t st = current_stream();
-  const double a = read_scalar_f64(alpha);
-  Mat c(C, accum == FaerV0_24_Accum_Add, st);
-  Mat lhs(A, st), rhs(B, st);
-  gemm_f64(st, c.s.view<double>(), RECT, accum == FaerV0_24_Accum_Add ? 1 : 0, lhs.s.view<const double>(), RECT,
-           rhs.s.view<const double>(), RECT, a);
-  finish_all(st, {&c.s, &lhs.s, &rhs.s});
-}
-
-void libfaer_v0_23_matmul_triangular_f64(FaerV0_24_MatMut C, FaerV0_24_Block C_block, FaerV0_24_Accum accum,
-                                         FaerV0_24_MatRef A, FaerV0_24_Block A_block, FaerV0_24_MatRef B,
-                                         FaerV0_24_Block B_block, const FaerV0_24_Scalar* alpha, FaerV0_24_Par par) {
-  (void)par;
-  FB_ENTRY();
-  FB_ASSERT(C.nrows == A.nrows && C.ncols == B.ncols && A.ncols == B.nrows, "matmul shape mismatch");
-  cudaStream_t st = current_stream();
-  const double a = read_scalar_f64(alpha);
-  const bool copy_in = accum == FaerV0_24_Accum_Add || C_block != FaerV0_24_Block_Rectangular;
-  Mat c(C, copy_in, st);
-  Mat lhs(A, st), rhs(B, st);
-  gemm_f64(st, c.s.view<double>(), (int)C_block, accum == FaerV0_24_Accum_Add ? 1 : 0, lhs.s.view<const double>(),
-           (int)A_block, rhs.s.view<const double>(), (int)B_block, a);
-  finish_all(st, {&c.s, &lhs.s, &rhs.s});
-}
-
-// ---- f32 matmul (3xTF32 tensor-core kernel) ----
-static void matmul_f32_impl(FaerV0_24_MatMut C, int C_block, FaerV0_24_Accum accum, FaerV0_24_MatRef A, int A_block,
-                            FaerV0_24_MatRef B, int B_block, const FaerV0_24_Scalar* alpha) {
-  FB_ENTRY();
-  FB_ASSERT(C.nrows == A.nrows && C.ncols == B.ncols && A.ncols == B.nrows, "matmul shape mismatch");
-  cudaStream_t st = current_stream();
-  FB_ASSERT(alpha != nullptr, "null scalar pointer");
-  float a;
-  if (is_device_pointer(alpha)) FB_CUDA_CHECK(cudaMemcpy(&a, alpha, 4, cudaMemcpyDeviceToHost));
-  else memcpy(&a, alpha, 4);
-  const bool copy_in = accum == FaerV0_24_Accum_Add || C_block != FaerV0_24_Block_Rectangular;
-  StagedMat c(C.ptr, (i64)C.nrows, (i64)C.ncols, (i64)C.row_stride, (i64)C.col_stride, 4, copy_in, true, st);
-  StagedMat l(A.ptr, (i64)A.nrows, (i64)A.ncols, (i64)A.row_stride, (i64)A.col_stride, 4, true, false, st);
-  StagedMat r(B.ptr, (i64)B.nrows, (i64)B.ncols, (i64)B.row_stride, (i64)B.col_stride, 4, true, false, st);
-  gemm_f32(st, c.view<float>(), C_block, accum == FaerV0_24_Accum_Add ? 1 : 0, l.view<const float>(), A_block,
-           r.view<const float>(), B_block, a);
-  finish_all(st, {&c, &l, &r});
-}
-void libfaer_v0_23_matmul_f32(FaerV0_24_MatMut C, FaerV0_24_Accum accum, FaerV0_24_MatRef A, FaerV0_24_MatRef B,
-                              const FaerV0_24_Scalar* alpha, FaerV0_24_Par par) {
-  (void)par;
-  matmul_f32_impl(C, 0, accum, A, 0, B, 0, alpha);
-}
-void libfaer_v0_23_matmul_triangular_f32(FaerV0_24_MatMut C, FaerV0_24_Block C_block, FaerV0_24_Accum accum,
-                                         FaerV0_24_MatRef A, FaerV0_24_Block A_block, FaerV0_24_MatRef B,
-                                         FaerV0_24_Block B_block, const FaerV0_24_Scalar* alpha, FaerV0_24_Par par) {
-  (void)par;
-  matmul_f32_impl(C, (int)C_block, accum, A, (int)A_block, B, (int)B_block, alpha);
-}
-
-// ---- c64 matmul (interleaved complex<f64>; `alpha` points to a complex scalar) ----
-static void matmul_c64_impl(FaerV0_24_MatMut C, int C_block, FaerV0_24_Accum accum, FaerV0_24_MatRef A, int A_block,
-                            FaerV0_24_MatRef B, int B_block, const FaerV0_24_Scalar* alpha, bool conj_a = false,
-                            bool conj_b = false) {
-  FB_ENTRY();
-  FB_ASSERT(C.nrows == A.nrows && C.ncols == B.ncols && A.ncols == B.nrows, "matmul shape mismatch");
-  cudaStream_t st = current_stream();
-  FB_ASSERT(alpha != nullptr, "null scalar pointer");
-  double a[2];
-  if (is_device_pointer(alpha)) FB_CUDA_CHECK(cudaMemcpy(a, alpha, 16, cudaMemcpyDeviceToHost));
-  else memcpy(a, alpha, 16);
-  const bool copy_in = accum == FaerV0_24_Accum_Add || C_block != FaerV0_24_Block_Rectangular;
-  StagedMat c(C.ptr, (i64)C.nrows, (i64)C.ncols, (i64)C.row_stride, (i64)C.col_stride, 16, copy_in, true, st);
-  StagedMat l(A.ptr, (i64)A.nrows, (i64)A.ncols, (i64)A.row_stride, (i64)A.col_stride, 16, true, false, st);
-  StagedMat r(B.ptr, (i64)B.nrows, (i64)B.ncols, (i64)B.row_stride, (i64)B.col_stride, 16, true, false, st);
-  // StagedMat views are in 16-byte element units; reinterpret the base as double* keeping complex strides
-  auto as_c = [](const StagedMat& s) { return s.view<double>(); };
-  VD dv = as_c(c);
-  VD lv0 = as_c(l), rv0 = as_c(r);
-  // view<double>() scaled pointer arithmetic by 8 bytes, but strides are in complex units: rebuild from the raw pointer
-  gemm_c64(st, dv, C_block, accum == FaerV0_24_Accum_Add ? 1 : 0, cv(lv0), A_block, conj_a, cv(rv0), B_block, conj_b, a[0],
-           a[1]);
-  finish_all(st, {&c, &l, &r});
-}
-void libfaer_v0_23_matmul_c64(FaerV0_24_MatMut C, FaerV0_24_Accum accum, FaerV0_24_MatRef A, FaerV0_24_MatRef B,
-                              const FaerV0_24_Scalar* alpha, FaerV0_24_Par par) {
-  (void)par;
-  matmul_c64_impl(C, 0, accum, A, 0, B, 0, alpha);
-}
-void libfaer_v0_23_matmul_triangular_c64(FaerV0_24_MatMut C, FaerV0_24_Block C_block, FaerV0_24_Accum accum,
-                                         FaerV0_24_MatRef A, FaerV0_24_Block A_block, FaerV0_24_MatRef B,
-                                         FaerV0_24_Block B_block, const FaerV0_24_Scalar* alpha, FaerV0_24_Par par) {
-  (void)par;
-  matmul_c64_impl(C, (int)C_block, accum, A, (int)A_block, B, (int)B_block, alpha);
-}
-
-static void matmul_c32_impl(FaerV0_24_MatMut C, int C_block, FaerV0_24_Accum accum, FaerV0_24_MatRef A, int A_block,
-                            FaerV0_24_MatRef B, int B_block, const FaerV0_24_Scalar* alpha, bool conj_a = false,
-                            bool conj_b = false) {
-  FB_ENTRY();
-  FB_ASSERT(C.nrows == A.nrows && C.ncols == B.ncols && A.ncols == B.nrows, "matmul shape mismatch");
-  cudaStream_t st = current_stream();
-  FB_ASSERT(alpha != nullptr, "null scalar pointer");
-  float a[2];
-  if (is_device_pointer(alpha)) FB_CUDA_CHECK(cudaMemcpy(a, alpha, 8, cudaMemcpyDeviceToHost));
-  else memcpy(a, alpha, 8);
-  const bool copy_in = accum == FaerV0_24_Accum_Add || C_block != FaerV0_24_Block_Rectangular;
-  // elements are 8-byte (re, im) pairs; the views keep strides in complex units and a float* base
-  StagedMat c(C.ptr, (i64)C.nrows, (i64)C.ncols, (i64)C.row_stride, (i64)C.col_stride, 8, copy_in, true, st);
-  StagedMat l(A.ptr, (i64)A.nrows, (i64)A.ncols, (i64)A.row_stride, (i64)A.col_stride, 8, true, false, st);
-  StagedMat r(B.ptr, (i64)B.nrows, (i64)B.ncols, (i64)B.row_stride, (i64)B.col_stride, 8, true, false, st);
-  VF dv = c.view<float>();
-  VF lv0 = l.view<float>(), rv0 = r.view<float>();
-  gemm_c32(st, dv, C_block, accum == FaerV0_24_Accum_Add ? 1 : 0, cv(lv0), A_block, conj_a, cv(rv0), B_block, conj_b, a[0],
-           a[1]);
-  finish_all(st, {&c, &l, &r});
-}
-void libfaer_v0_23_matmul_c32(FaerV0_24_MatMut C, FaerV0_24_Accum accum, FaerV0_24_MatRef A, FaerV0_24_MatRef B,
-                              const FaerV0_24_Scalar* alpha, FaerV0_24_Par par) {
-  (void)par;
-  matmul_c32_impl(C, 0, accum, A, 0, B, 0, alpha);
-}
-void libfaer_v0_23_matmul_triangular_c32(FaerV0_24_MatMut C, FaerV0_24_Block C_block, FaerV0_24_Accum accum,
-                                         FaerV0_24_MatRef A, FaerV0_24_Block A_block, FaerV0_24_MatRef B,
-                                         FaerV0_24_Block B_block, const FaerV0_24_Scalar* alpha, FaerV0_24_Par par) {
-  (void)par;
-  matmul_c32_impl(C, (int)C_block, accum, A, (int)A_block, B, (int)B_block, alpha);
-}
-
-#define FB_TRSM_FFI(SUF, T)                                                                                            \
-  void libfaer_v0_23_solve_triangular_lower_in_place_##SUF(FaerV0_24_MatRef L, FaerV0_24_Conj L_conj, FaerV0_24_MatMut rhs, \
-                                                           FaerV0_24_Par par) {                                        \
-    (void)L_conj; (void)par;                                                                                           \
-    solve_tri<T>(L, rhs, true, false);                                                                                 \
-  }                                                                                                                    \
-  void libfaer_v0_23_solve_triangular_upper_in_place_##SUF(FaerV0_24_MatRef U, FaerV0_24_Conj U_conj, FaerV0_24_MatMut rhs, \
-                                                           FaerV0_24_Par par) {                                        \
-    (void)U_conj; (void)par;                                                                                           \
-    solve_tri<T>(U, rhs, false, false);                                                                                \
-  }                                                                                                                    \
-  void libfaer_v0_23_solve_unit_triangular_lower_in_place_##SUF(FaerV0_24_MatRef L, FaerV0_24_Conj L_conj,             \
-                                                                FaerV0_24_MatMut rhs, FaerV0_24_Par par) {             \
-    (void)L_conj; (void)par;                                                                                           \
-    solve_tri<T>(L, rhs, true, true);                                                                                  \
-  }                                                                                                                    \
-  void libfaer_v0_23_solve_unit_triangular_upper_in_place_##SUF(FaerV0_24_MatRef U, FaerV0_24_Conj U_conj,             \
-                                                                FaerV0_24_MatMut rhs, FaerV0_24_Par par) {             \
-    (void)U_conj; (void)par;                                                                                           \
-    solve_tri<T>(U, rhs, false, true);                                                                                 \
+// ---- matmul ----
+#define FB_MATMUL_FFI(SUF, R, CX)                                                                                               \
+  void libfaer_v0_23_matmul_##SUF(FaerV0_24_MatMut C, FaerV0_24_Accum accum, FaerV0_24_MatRef A, FaerV0_24_MatRef B,            \
+                                  const FaerV0_24_Scalar* alpha, FaerV0_24_Par par) {                                           \
+    (void)par;                                                                                                                  \
+    matmul_entry<R, CX>(C, RECT, accum, A, RECT, B, RECT, alpha);                                                               \
+  }                                                                                                                             \
+  void libfaer_v0_23_matmul_triangular_##SUF(FaerV0_24_MatMut C, FaerV0_24_Block C_block, FaerV0_24_Accum accum,                \
+                                             FaerV0_24_MatRef A, FaerV0_24_Block A_block, FaerV0_24_MatRef B,                   \
+                                             FaerV0_24_Block B_block, const FaerV0_24_Scalar* alpha, FaerV0_24_Par par) {       \
+    (void)par;                                                                                                                  \
+    matmul_entry<R, CX>(C, (int)C_block, accum, A, (int)A_block, B, (int)B_block, alpha);                                       \
   }
-FB_TRSM_FFI(f64, double)
-FB_TRSM_FFI(f32, float)
+FB_MATMUL_FFI(f64, double, false)
+FB_MATMUL_FFI(f32, float, false)
+FB_MATMUL_FFI(c64, double, true)
+FB_MATMUL_FFI(c32, float, true)
+#undef FB_MATMUL_FFI
+
+// ---- triangular solves ----
+#define FB_TRSM_FFI(SUF, R, CX)                                                                                                 \
+  void libfaer_v0_23_solve_triangular_lower_in_place_##SUF(FaerV0_24_MatRef L, FaerV0_24_Conj L_conj, FaerV0_24_MatMut rhs,     \
+                                                           FaerV0_24_Par par) {                                                 \
+    (void)par;                                                                                                                  \
+    solve_tri_entry<R, CX>(L, L_conj, rhs, true, false);                                                                        \
+  }                                                                                                                             \
+  void libfaer_v0_23_solve_triangular_upper_in_place_##SUF(FaerV0_24_MatRef U, FaerV0_24_Conj U_conj, FaerV0_24_MatMut rhs,     \
+                                                           FaerV0_24_Par par) {                                                 \
+    (void)par;                                                                                                                  \
+    solve_tri_entry<R, CX>(U, U_conj, rhs, false, false);                                                                       \
+  }                                                                                                                             \
+  void libfaer_v0_23_solve_unit_triangular_lower_in_place_##SUF(FaerV0_24_MatRef L, FaerV0_24_Conj L_conj, FaerV0_24_MatMut rhs, \
+                                                                FaerV0_24_Par par) {                                            \
+    (void)par;                                                                                                                  \
+    solve_tri_entry<R, CX>(L, L_conj, rhs, true, true);                                                                         \
+  }                                                                                                                             \
+  void libfaer_v0_23_solve_unit_triangular_upper_in_place_##SUF(FaerV0_24_MatRef U, FaerV0_24_Conj U_conj, FaerV0_24_MatMut rhs, \
+                                                                FaerV0_24_Par par) {                                            \
+    (void)par;                                                                                                                  \
+    solve_tri_entry<R, CX>(U, U_conj, rhs, false, true);                                                                        \
+  }
+FB_TRSM_FFI(f64, double, false)
+FB_TRSM_FFI(f32, float, false)
+FB_TRSM_FFI(c64, double, true)
+FB_TRSM_FFI(c32, float, true)
 #undef FB_TRSM_FFI
 
 // ---- LLT ----
-FaerV0_24_LltParams libfaer_v0_23_LltParams_f64(void) {
-  // reference defaults: faer/src/linalg/cholesky/ldlt/factor.rs:705-714
-  return FaerV0_24_LltParams{64, 128};
-}
-
-FaerV0_24_Layout libfaer_v0_23_llt_factor_in_place_scratch_f64(size_t dim, FaerV0_24_Par par,
-                                                               FaerV0_24_LltParams params) {
-  (void)par; (void)params;
-  // reference: temp_mat_scratch::<T>(dim, 1) (llt/factor.rs:58-66). The GPU path keeps its (tiny) workspace in
-  // the internal device pool, but reports the reference's requirement so callers allocate identically.
-  return FaerV0_24_Layout{dim * sizeof(double), 64};
-}
-
-FaerV0_24_LltStatus libfaer_v0_23_llt_factor_in_place_f64(FaerV0_24_MatMut A, FaerV0_24_LltRegularization regularization,
-                                                          FaerV0_24_Par par, FaerV0_24_MemAlloc mem,
-                                                          FaerV0_24_LltParams params) {
-  (void)par; (void)mem;
-  FB_ENTRY();
-  FB_ASSERT(A.nrows == A.ncols, "LLT needs a square matrix");
-  cudaStream_t st = current_stream();
-  double delta = 0.0, eps = 0.0;
-  if (regularization.dynamic_regularization_delta)
-    delta = read_scalar_f64((const FaerV0_24_Scalar*)regularization.dynamic_regularization_delta);
-  if (regularization.dynamic_regularization_epsilon)
-    eps = read_scalar_f64((const FaerV0_24_Scalar*)regularization.dynamic_regularization_epsilon);
-  LltResult r;
-  if (A.nrows > 0 && !is_device_pointer(A.ptr) && A.row_stride == 1 && A.col_stride >= (ptrdiff_t)A.nrows &&
-      (i64)A.nrows >= lookahead_min_n()) {
-    // host matrix: upload / factor / download pipelined block column by block column (dist.cu)
-    FB_CUDA_CHECK(cudaStreamSynchronize(st));
-    const i64 nb = lookahead_block() ? lookahead_block() : 256;
-    r = llt_host_pipelined_f64((double*)A.ptr, (i64)A.col_stride, (i64)A.nrows, nb, delta, eps);
-  } else {
-    Mat a(A, true, st);
-    r = llt_cholesky_in_place_f64(st, a.s.view<double>(), delta, eps,
-                                  LltParams{params.recursion_threshold, params.block_size});
-    finish_all(st, {&a.s});
+// the GPU path keeps its (tiny) workspace in the internal device pool, but reports the reference's requirement so callers allocate
+// identically
+#define FB_LLT_QUERIES(SUF, ES)                                                                                                 \
+  FaerV0_24_LltParams libfaer_v0_23_LltParams_##SUF(void) { return FaerV0_24_LltParams{64, 128}; /* ldlt/factor.rs:705-714 */ } \
+  FaerV0_24_Layout libfaer_v0_23_llt_factor_in_place_scratch_##SUF(size_t dim, FaerV0_24_Par par, FaerV0_24_LltParams params) { \
+    (void)par; (void)params;                                                                                                    \
+    return FaerV0_24_Layout{dim * (ES), 64}; /* temp_mat_scratch::<T>(dim, 1), llt/factor.rs:58-66 */                           \
+  }                                                                                                                             \
+  FaerV0_24_Layout libfaer_v0_23_llt_solve_in_place_scratch_##SUF(size_t dim, size_t rhs_ncols, FaerV0_24_Par par) {            \
+    (void)dim; (void)rhs_ncols; (void)par;                                                                                      \
+    return FaerV0_24_Layout{0, 1}; /* StackReq::EMPTY (llt/solve.rs:3-10) */                                                    \
   }
-  FaerV0_24_LltStatus out;
-  memset(&out, 0, sizeof(out));
-  if (r.ok) {
-    out.tag = FaerV0_24_LltStatus_Ok;
-    out.ok.dynamic_regularization_count = r.dynamic_regularization_count;
-  } else {
-    out.tag = FaerV0_24_LltStatus_NonPositivePivot;
-    out.non_positive_pivot.index = r.non_positive_pivot_index;
+#define FB_LLT_FFI(SUF, R, CX)                                                                                                  \
+  FaerV0_24_LltStatus libfaer_v0_23_llt_factor_in_place_##SUF(FaerV0_24_MatMut A, FaerV0_24_LltRegularization regularization,   \
+                                                              FaerV0_24_Par par, FaerV0_24_MemAlloc mem,                        \
+                                                              FaerV0_24_LltParams params) {                                     \
+    (void)par; (void)mem;                                                                                                       \
+    return llt_factor_entry<R, CX>(A, regularization, params);                                                                  \
+  }                                                                                                                             \
+  void libfaer_v0_23_llt_solve_in_place_##SUF(FaerV0_24_MatRef L, FaerV0_24_Conj A_conj, FaerV0_24_MatMut rhs,                  \
+                                              FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {                                      \
+    (void)par; (void)mem;                                                                                                       \
+    llt_solve_entry<R, CX>(L, A_conj, rhs);                                                                                     \
   }
-  return out;
-}
+FB_LLT_QUERIES(f64, sizeof(double))
+FB_LLT_QUERIES(f32, sizeof(float))
+FB_LLT_QUERIES(c64, 2 * sizeof(double))
+FB_LLT_QUERIES(c32, 2 * sizeof(float))
+FB_LLT_FFI(f64, double, false)
+FB_LLT_FFI(f32, float, false)
+FB_LLT_FFI(c64, double, true)
+FB_LLT_FFI(c32, float, true)
+#undef FB_LLT_QUERIES
+#undef FB_LLT_FFI
 
-// ---- f32 LLT (llt.cu: the templated leaf kernel and recursive driver instantiated for float) ----
-static float read_real_f32(const void* p) {
-  float v;
-  if (is_device_pointer(p)) FB_CUDA_CHECK(cudaMemcpy(&v, p, sizeof(float), cudaMemcpyDeviceToHost));
-  else memcpy(&v, p, sizeof(float));
-  return v;
-}
-FaerV0_24_LltParams libfaer_v0_23_LltParams_f32(void) { return FaerV0_24_LltParams{64, 128}; }
-FaerV0_24_Layout libfaer_v0_23_llt_factor_in_place_scratch_f32(size_t dim, FaerV0_24_Par par, FaerV0_24_LltParams params) {
-  (void)par; (void)params;
-  return FaerV0_24_Layout{dim * sizeof(float), 64};  // temp_mat_scratch::<T>(dim, 1), llt/factor.rs:58-66
-}
-FaerV0_24_LltStatus libfaer_v0_23_llt_factor_in_place_f32(FaerV0_24_MatMut A, FaerV0_24_LltRegularization regularization,
-                                                          FaerV0_24_Par par, FaerV0_24_MemAlloc mem,
-                                                          FaerV0_24_LltParams params) {
-  (void)par; (void)mem;
-  FB_ENTRY();
-  FB_ASSERT(A.nrows == A.ncols, "LLT needs a square matrix");
-  cudaStream_t st = current_stream();
-  float delta = 0.0f, eps = 0.0f;
-  if (regularization.dynamic_regularization_delta) delta = read_real_f32(regularization.dynamic_regularization_delta);
-  if (regularization.dynamic_regularization_epsilon) eps = read_real_f32(regularization.dynamic_regularization_epsilon);
-  StagedMat a(A.ptr, (i64)A.nrows, (i64)A.ncols, (i64)A.row_stride, (i64)A.col_stride, sizeof(float), true, true, st);
-  const LltResult r = llt_cholesky_in_place_f32(st, a.view<float>(), delta, eps,
-                                                LltParams{params.recursion_threshold, params.block_size});
-  finish_all(st, {&a});
-  FaerV0_24_LltStatus out;
-  memset(&out, 0, sizeof(out));
-  if (r.ok) {
-    out.tag = FaerV0_24_LltStatus_Ok;
-    out.ok.dynamic_regularization_count = r.dynamic_regularization_count;
-  } else {
-    out.tag = FaerV0_24_LltStatus_NonPositivePivot;
-    out.non_positive_pivot.index = r.non_positive_pivot_index;
-  }
-  return out;
-}
-FaerV0_24_Layout libfaer_v0_23_llt_solve_in_place_scratch_f32(size_t dim, size_t rhs_ncols, FaerV0_24_Par par) {
-  (void)dim; (void)rhs_ncols; (void)par;
-  return FaerV0_24_Layout{0, 1};
-}
-void libfaer_v0_23_llt_solve_in_place_f32(FaerV0_24_MatRef L, FaerV0_24_Conj A_conj, FaerV0_24_MatMut rhs, FaerV0_24_Par par,
-                                          FaerV0_24_MemAlloc mem) {
-  (void)A_conj; (void)par; (void)mem;
-  FB_ENTRY();
-  cudaStream_t st = current_stream();
-  FB_ASSERT(L.nrows == L.ncols && rhs.nrows == L.nrows, "LLT solve shape mismatch");
-  StagedMat l(L.ptr, (i64)L.nrows, (i64)L.ncols, (i64)L.row_stride, (i64)L.col_stride, sizeof(float), true, false, st);
-  StagedMat r(rhs.ptr, (i64)rhs.nrows, (i64)rhs.ncols, (i64)rhs.row_stride, (i64)rhs.col_stride, sizeof(float), true, true, st);
-  llt_solve_in_place_f32(st, l.view<const float>(), r.view<float>());
-  finish_all(st, {&l, &r});
-}
-
-// ---- LDLT (no pivoting), f64: ldlt_f64.cu (the other dtypes, reconstruct and inverse: ffi_types.cu / ldlt_types.cu) ----
-FaerV0_24_LdltParams libfaer_v0_23_LdltParams_f64(void) {
-  return FaerV0_24_LdltParams{64, 128};  // reference defaults: ldlt/factor.rs:705-714
-}
-FaerV0_24_Layout libfaer_v0_23_ldlt_factor_in_place_scratch_f64(size_t dim, FaerV0_24_Par par, FaerV0_24_LdltParams params) {
-  (void)par; (void)params;
-  return FaerV0_24_Layout{dim * sizeof(double), 64};  // temp_mat_scratch::<T>(dim, 1), ldlt/factor.rs:715-724
-}
+// ---- LDLT (no pivoting), f64: ldlt_f64.cu (the other dtypes, reconstruct, inverse and the queries: ffi_types.cu) ----
 FaerV0_24_LdltStatus libfaer_v0_23_ldlt_factor_in_place_f64(FaerV0_24_MatMut A, FaerV0_24_LdltRegularization regularization,
                                                             FaerV0_24_Par par, FaerV0_24_MemAlloc mem,
                                                             FaerV0_24_LdltParams params) {
@@ -647,44 +447,14 @@ FaerV0_24_LdltStatus libfaer_v0_23_ldlt_factor_in_place_f64(FaerV0_24_MatMut A, 
   FB_ENTRY();
   FB_ASSERT(A.nrows == A.ncols, "LDLT needs a square matrix");
   cudaStream_t st = current_stream();
-  double delta = 0.0, eps = 0.0;
-  if (regularization.dynamic_regularization_delta)
-    delta = read_scalar_f64((const FaerV0_24_Scalar*)regularization.dynamic_regularization_delta);
-  if (regularization.dynamic_regularization_epsilon)
-    eps = read_scalar_f64((const FaerV0_24_Scalar*)regularization.dynamic_regularization_epsilon);
-  // expected signs: i8 slice, null = none (faer-ffi/src/lib.rs:838-848); host slices are mirrored on the device
-  const signed char* d_signs = nullptr;
-  signed char* signs_mirror = nullptr;
-  const FaerV0_24_SliceMut sg = regularization.dynamic_regularization_signs;
-  if (sg.ptr != nullptr && A.nrows > 0) {
-    FB_ASSERT(sg.len >= A.nrows, "dynamic_regularization_signs is shorter than the matrix dimension");
-    if (is_device_pointer(sg.ptr)) {
-      d_signs = (const signed char*)sg.ptr;
-    } else {
-      signs_mirror = (signed char*)ws_alloc(A.nrows);
-      FB_CUDA_CHECK(cudaMemcpyAsync(signs_mirror, sg.ptr, A.nrows, cudaMemcpyHostToDevice, st));
-      d_signs = signs_mirror;
-    }
-  }
-  Mat a(A, true, st);
-  const LdltResult r = ldlt_in_place_f64(st, a.s.view<double>(), delta, eps, d_signs,
+  double delta, eps;
+  read_regularization(regularization, delta, eps);
+  const SignsArg signs(regularization.dynamic_regularization_signs, A.nrows, st);
+  StagedMat a = stage(A, sizeof(double), true, st);
+  const LdltResult r = ldlt_in_place_f64(st, a.view<double>(), delta, eps, signs.ptr,
                                          LltParams{params.recursion_threshold, params.block_size});
-  finish_all(st, {&a.s});
-  if (signs_mirror) ws_free(signs_mirror);
-  FaerV0_24_LdltStatus out;
-  memset(&out, 0, sizeof(out));
-  if (r.ok) {
-    out.tag = FaerV0_24_LdltStatus_Ok;
-    out.ok.dynamic_regularization_count = r.dynamic_regularization_count;
-  } else {
-    out.tag = FaerV0_24_LdltStatus_ZeroPivot;
-    out.zero_pivot.index = r.zero_pivot_index;
-  }
-  return out;
-}
-FaerV0_24_Layout libfaer_v0_23_ldlt_solve_in_place_scratch_f64(size_t dim, size_t rhs_ncols, FaerV0_24_Par par) {
-  (void)dim; (void)rhs_ncols; (void)par;
-  return FaerV0_24_Layout{0, 1};  // StackReq::EMPTY (ldlt/solve.rs:3-10)
+  finish_all(st, {&a});
+  return ldlt_status(r);
 }
 void libfaer_v0_23_ldlt_solve_in_place_f64(FaerV0_24_MatRef L, FaerV0_24_VecRef D, FaerV0_24_Conj A_conj, FaerV0_24_MatMut rhs,
                                            FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {
@@ -694,275 +464,73 @@ void libfaer_v0_23_ldlt_solve_in_place_f64(FaerV0_24_MatRef L, FaerV0_24_VecRef 
   const size_t n = L.nrows;
   FB_ASSERT(L.ncols == n && D.len == n && rhs.nrows == n, "LDLT solve shape mismatch");
   if (n == 0 || rhs.ncols == 0) return;
-  Mat l(L, st);
-  Mat r(rhs, true, st);
-  // D: usually the diagonal of the factored matrix (stride = row_stride + col_stride). A host vector is gathered into a
-  // compact device copy; a device vector is read in place.
-  const double* d_ptr = (const double*)D.ptr;
-  i64 d_stride = (i64)D.stride;
-  double* d_mirror = nullptr;
-  if (!is_device_pointer(D.ptr)) {
-    std::vector<double> h(n);
-    for (size_t i = 0; i < n; ++i) h[i] = ((const double*)D.ptr)[(ptrdiff_t)i * D.stride];
-    d_mirror = (double*)ws_alloc(n * sizeof(double));
-    FB_CUDA_CHECK(cudaMemcpyAsync(d_mirror, h.data(), n * sizeof(double), cudaMemcpyHostToDevice, st));
-    FB_CUDA_CHECK(cudaStreamSynchronize(st));  // `h` is pageable and local
-    d_ptr = d_mirror;
-    d_stride = 1;
-  }
-  ldlt_solve_in_place_f64(st, l.s.view<const double>(), d_ptr, d_stride, r.s.view<double>());
-  finish_all(st, {&l.s, &r.s});
-  if (d_mirror) ws_free(d_mirror);
+  StagedMat l = stage(L, sizeof(double), st), r = stage(rhs, sizeof(double), true, st);
+  // D: usually the diagonal of the factored matrix (stride = row_stride + col_stride)
+  const DiagArg<double, false> d(D, n, st);
+  ldlt_solve_in_place_f64(st, l.view<const double>(), d.ptr, d.stride, r.view<double>());
+  finish_all(st, {&l, &r});
 }
-
-// ---- c64 / c32 triangular solves and LLT (cplx.cu: faer's recursions on the complex GEMMs + scalar complex leaf kernels) ----
-#define FB_CPLX_TRSM_LLT(SUF, R)                                                                                                \
-  void libfaer_v0_23_solve_triangular_lower_in_place_##SUF(FaerV0_24_MatRef L, FaerV0_24_Conj L_conj, FaerV0_24_MatMut rhs,     \
-                                                           FaerV0_24_Par par) {                                                 \
-    (void)par;                                                                                                                  \
-    solve_tri_cplx<R>(L, L_conj, rhs, true, false);                                                                             \
-  }                                                                                                                             \
-  void libfaer_v0_23_solve_triangular_upper_in_place_##SUF(FaerV0_24_MatRef U, FaerV0_24_Conj U_conj, FaerV0_24_MatMut rhs,     \
-                                                           FaerV0_24_Par par) {                                                 \
-    (void)par;                                                                                                                  \
-    solve_tri_cplx<R>(U, U_conj, rhs, false, false);                                                                            \
-  }                                                                                                                             \
-  void libfaer_v0_23_solve_unit_triangular_lower_in_place_##SUF(FaerV0_24_MatRef L, FaerV0_24_Conj L_conj, FaerV0_24_MatMut rhs, \
-                                                                FaerV0_24_Par par) {                                            \
-    (void)par;                                                                                                                  \
-    solve_tri_cplx<R>(L, L_conj, rhs, true, true);                                                                              \
-  }                                                                                                                             \
-  void libfaer_v0_23_solve_unit_triangular_upper_in_place_##SUF(FaerV0_24_MatRef U, FaerV0_24_Conj U_conj, FaerV0_24_MatMut rhs, \
-                                                                FaerV0_24_Par par) {                                            \
-    (void)par;                                                                                                                  \
-    solve_tri_cplx<R>(U, U_conj, rhs, false, true);                                                                             \
-  }                                                                                                                             \
-  FaerV0_24_LltParams libfaer_v0_23_LltParams_##SUF(void) { return FaerV0_24_LltParams{64, 128}; }                              \
-  FaerV0_24_Layout libfaer_v0_23_llt_factor_in_place_scratch_##SUF(size_t dim, FaerV0_24_Par par, FaerV0_24_LltParams params) { \
-    (void)par; (void)params;                                                                                                    \
-    return FaerV0_24_Layout{dim * 2 * sizeof(R), 64}; /* temp_mat_scratch::<T>(dim, 1), llt/factor.rs:58-66 */                  \
-  }                                                                                                                             \
-  FaerV0_24_LltStatus libfaer_v0_23_llt_factor_in_place_##SUF(FaerV0_24_MatMut A, FaerV0_24_LltRegularization regularization,   \
-                                                              FaerV0_24_Par par, FaerV0_24_MemAlloc mem,                        \
-                                                              FaerV0_24_LltParams params) {                                     \
-    (void)par; (void)mem; (void)params;                                                                                         \
-    return llt_factor_cplx<R>(A, regularization);                                                                               \
-  }                                                                                                                             \
-  FaerV0_24_Layout libfaer_v0_23_llt_solve_in_place_scratch_##SUF(size_t dim, size_t rhs_ncols, FaerV0_24_Par par) {            \
-    (void)dim; (void)rhs_ncols; (void)par;                                                                                      \
-    return FaerV0_24_Layout{0, 1};                                                                                              \
-  }                                                                                                                             \
-  void libfaer_v0_23_llt_solve_in_place_##SUF(FaerV0_24_MatRef L, FaerV0_24_Conj A_conj, FaerV0_24_MatMut rhs,                  \
-                                              FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {                                      \
-    (void)par; (void)mem;                                                                                                       \
-    llt_solve_cplx<R>(L, A_conj, rhs);                                                                                          \
-  }
-FB_CPLX_TRSM_LLT(c64, double)
-FB_CPLX_TRSM_LLT(c32, float)
-#undef FB_CPLX_TRSM_LLT
 
 // ---- partial-pivoting LU ----
-FaerV0_24_PartialPivLuParams libfaer_v0_23_PartialPivLuParams_f64(void) {
-  // reference defaults: faer/src/linalg/lu/partial_pivoting/factor.rs:212-222
-  return FaerV0_24_PartialPivLuParams{16, 64, 128 * 128};
-}
-
-static FaerV0_24_Layout lu_scratch(size_t nrows, size_t ncols, size_t idx_bytes) {
-  // reference: StackReq::new::<I>(min(nrows, ncols)) (factor.rs:224-233)
-  size_t size = nrows < ncols ? nrows : ncols;
-  return FaerV0_24_Layout{size * idx_bytes, idx_bytes};
-}
-FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_factor_in_place_scratch_u32_f64(size_t nrows, size_t ncols, FaerV0_24_Par par,
-                                                                              FaerV0_24_PartialPivLuParams params) {
-  (void)par; (void)params;
-  return lu_scratch(nrows, ncols, 4);
-}
-FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_factor_in_place_scratch_u64_f64(size_t nrows, size_t ncols, FaerV0_24_Par par,
-                                                                              FaerV0_24_PartialPivLuParams params) {
-  (void)par; (void)params;
-  return lu_scratch(nrows, ncols, 8);
-}
-
-static FaerV0_24_PartialPivLuStatus lu_entry(FaerV0_24_MatMut A, FaerV0_24_SliceMut perm_fwd, FaerV0_24_SliceMut perm_bwd,
-                                             FaerV0_24_PartialPivLuParams params, int idx_bytes) {
-  FB_ENTRY();
-  cudaStream_t st = current_stream();
-  // NB: faer.hpp fills SliceMut.len with BYTES while the Rust side reads elements (SURVEY.md appendix A), so the
-  // permutation length is taken from A.nrows, never from `len`.
-  FB_ASSERT(A.nrows == 0 || (perm_fwd.ptr != nullptr && perm_bwd.ptr != nullptr), "null permutation slice");
-  Mat a(A, true, st);
-  size_t cnt = lu_partial_piv_in_place_f64(st, a.s.view<double>(), perm_fwd.ptr, perm_bwd.ptr, idx_bytes,
-                                           PartialPivLuParams{params.recursion_threshold, params.block_size,
-                                                              params.par_threshold});
-  finish_all(st, {&a.s});
-  FaerV0_24_PartialPivLuStatus out;
-  memset(&out, 0, sizeof(out));
-  out.tag = FaerV0_24_PartialPivLuStatus_Ok;
-  out.ok.transposition_count = cnt;
-  return out;
-}
-FaerV0_24_PartialPivLuStatus libfaer_v0_23_partial_piv_lu_factor_in_place_u32_f64(
-    FaerV0_24_MatMut A, FaerV0_24_SliceMut perm_fwd, FaerV0_24_SliceMut perm_bwd, FaerV0_24_Par par, FaerV0_24_MemAlloc mem,
-    FaerV0_24_PartialPivLuParams params) {
-  (void)par; (void)mem;
-  return lu_entry(A, perm_fwd, perm_bwd, params, 4);
-}
-FaerV0_24_PartialPivLuStatus libfaer_v0_23_partial_piv_lu_factor_in_place_u64_f64(
-    FaerV0_24_MatMut A, FaerV0_24_SliceMut perm_fwd, FaerV0_24_SliceMut perm_bwd, FaerV0_24_Par par, FaerV0_24_MemAlloc mem,
-    FaerV0_24_PartialPivLuParams params) {
-  (void)par; (void)mem;
-  return lu_entry(A, perm_fwd, perm_bwd, params, 8);
-}
-
-// ---- f32 partial-pivoting LU: computed in f64, like the f32 `svd` / `self_adjoint_evd`. The f32 matrix is widened on the
-// device, factored by the f64 drivers (fused sub-panel kernel, TMA-fed GEMM, SM partition) and rounded back: the factors carry
-// one f32 rounding instead of an f32 elimination's accumulated ones, and the pivot search sees f64 values (so a pivot can
-// differ from an all-f32 elimination's where two candidates agree to f32 precision — either choice is a valid partial
-// pivot). The solves run on the native f32 triangular solves.
-FaerV0_24_PartialPivLuParams libfaer_v0_23_PartialPivLuParams_f32(void) { return libfaer_v0_23_PartialPivLuParams_f64(); }
-FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_factor_in_place_scratch_u32_f32(size_t nrows, size_t ncols, FaerV0_24_Par par,
-                                                                              FaerV0_24_PartialPivLuParams params) {
-  (void)par; (void)params;
-  return lu_scratch(nrows, ncols, 4);
-}
-FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_factor_in_place_scratch_u64_f32(size_t nrows, size_t ncols, FaerV0_24_Par par,
-                                                                              FaerV0_24_PartialPivLuParams params) {
-  (void)par; (void)params;
-  return lu_scratch(nrows, ncols, 8);
-}
-static FaerV0_24_PartialPivLuStatus lu_entry_f32(FaerV0_24_MatMut A, FaerV0_24_SliceMut perm_fwd, FaerV0_24_SliceMut perm_bwd,
-                                                 FaerV0_24_PartialPivLuParams params, int idx_bytes) {
-  FB_ENTRY();
-  cudaStream_t st = current_stream();
-  FB_ASSERT(A.nrows == 0 || (perm_fwd.ptr != nullptr && perm_bwd.ptr != nullptr), "null permutation slice");
-  const i64 m = (i64)A.nrows, n = (i64)A.ncols;
-  StagedMat a(A.ptr, m, n, (i64)A.row_stride, (i64)A.col_stride, 4, true, true, st);
-  VF av = a.view<float>();
-  const i64 ld = std::max<i64>(1, (m + 1) & ~(i64)1);
-  double* W = (double*)ws_alloc((size_t)ld * (size_t)std::max<i64>(n, 1) * 8);
-  ffi_cast<double, float>(st, W, 1, ld, av.ptr, av.rs, av.cs, m, n);
-  const size_t cnt = lu_partial_piv_in_place_f64(st, VD{W, m, n, 1, ld}, perm_fwd.ptr, perm_bwd.ptr, idx_bytes,
-                                                 PartialPivLuParams{params.recursion_threshold, params.block_size,
-                                                                    params.par_threshold});
-  ffi_cast<float, double>(st, av.ptr, av.rs, av.cs, W, 1, ld, m, n);
-  finish_all(st, {&a});
-  ws_free(W);
-  FaerV0_24_PartialPivLuStatus out;
-  memset(&out, 0, sizeof(out));
-  out.tag = FaerV0_24_PartialPivLuStatus_Ok;
-  out.ok.transposition_count = cnt;
-  return out;
-}
-FaerV0_24_PartialPivLuStatus libfaer_v0_23_partial_piv_lu_factor_in_place_u32_f32(
-    FaerV0_24_MatMut A, FaerV0_24_SliceMut perm_fwd, FaerV0_24_SliceMut perm_bwd, FaerV0_24_Par par, FaerV0_24_MemAlloc mem,
-    FaerV0_24_PartialPivLuParams params) {
-  (void)par; (void)mem;
-  return lu_entry_f32(A, perm_fwd, perm_bwd, params, 4);
-}
-FaerV0_24_PartialPivLuStatus libfaer_v0_23_partial_piv_lu_factor_in_place_u64_f32(
-    FaerV0_24_MatMut A, FaerV0_24_SliceMut perm_fwd, FaerV0_24_SliceMut perm_bwd, FaerV0_24_Par par, FaerV0_24_MemAlloc mem,
-    FaerV0_24_PartialPivLuParams params) {
-  (void)par; (void)mem;
-  return lu_entry_f32(A, perm_fwd, perm_bwd, params, 8);
-}
-
-// ---- Householder QR (no pivoting) + block-Householder sequence application, f64 and f32 (helpers above) ----
-#define FB_QR_FFI(SUF, T)                                                                                              \
-  FaerV0_24_QrParams libfaer_v0_23_QrParams_##SUF(void) { return FaerV0_24_QrParams{48 * 48, 192 * 256}; }             \
-  size_t libfaer_v0_23_qr_recommended_block_size_##SUF(size_t nrows, size_t ncols) {                                   \
-    return (size_t)qr_recommended_block_size((i64)nrows, (i64)ncols);                                                  \
-  }                                                                                                                    \
-  FaerV0_24_Layout libfaer_v0_23_qr_factor_in_place_scratch_##SUF(size_t nrows, size_t ncols, size_t block_size,       \
-                                                                  FaerV0_24_Par par, FaerV0_24_QrParams params) {      \
-    (void)nrows; (void)par; (void)params;                                                                              \
-    return FaerV0_24_Layout{block_size * ncols * sizeof(T), 64}; /* temp_mat_scratch(block_size, ncols) */            \
-  }                                                                                                                    \
-  FaerV0_24_QrStatus libfaer_v0_23_qr_factor_in_place_##SUF(FaerV0_24_MatMut A, FaerV0_24_MatMut Q_coeff, FaerV0_24_Par par, \
-                                                            FaerV0_24_MemAlloc mem, FaerV0_24_QrParams params) {       \
-    (void)par; (void)mem; (void)params;                                                                                \
-    return qr_entry<T>(A, Q_coeff);                                                                                    \
-  }                                                                                                                    \
-  FaerV0_24_Layout libfaer_v0_23_apply_householder_on_the_left_scratch_##SUF(size_t dim, size_t block_size, size_t rhs_ncols) { \
-    (void)dim;                                                                                                         \
-    return FaerV0_24_Layout{block_size * rhs_ncols * sizeof(T), 64};                                                   \
-  }                                                                                                                    \
-  FaerV0_24_Layout libfaer_v0_23_apply_householder_transpose_on_the_left_scratch_##SUF(size_t dim, size_t block_size,  \
-                                                                                        size_t rhs_ncols) {            \
-    (void)dim;                                                                                                         \
-    return FaerV0_24_Layout{block_size * rhs_ncols * sizeof(T), 64};                                                   \
-  }                                                                                                                    \
-  void libfaer_v0_23_apply_householder_on_the_left_##SUF(FaerV0_24_MatRef basis, FaerV0_24_MatRef factor, FaerV0_24_Conj conj, \
-                                                         FaerV0_24_MatMut rhs, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) { \
-    (void)conj; (void)par; (void)mem;                                                                                  \
-    householder_seq_entry<T>(basis, factor, rhs, false);                                                               \
-  }                                                                                                                    \
-  void libfaer_v0_23_apply_householder_transpose_on_the_left_##SUF(FaerV0_24_MatRef basis, FaerV0_24_MatRef factor,    \
-                                                                   FaerV0_24_Conj conj, FaerV0_24_MatMut rhs,          \
-                                                                   FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {        \
-    (void)conj; (void)par; (void)mem;                                                                                  \
-    householder_seq_entry<T>(basis, factor, rhs, true);                                                                \
-  }                                                                                                                    \
-  /* on the right = the transposed sequence on the left of the transposed view, and vice versa (householder.rs:813-854) */ \
-  FaerV0_24_Layout libfaer_v0_23_apply_householder_on_the_right_scratch_##SUF(size_t dim, size_t block_size, size_t lhs_nrows) { \
-    (void)dim;                                                                                                         \
-    return FaerV0_24_Layout{block_size * lhs_nrows * sizeof(T), 64};                                                   \
-  }                                                                                                                    \
-  FaerV0_24_Layout libfaer_v0_23_apply_householder_transpose_on_the_right_scratch_##SUF(size_t dim, size_t block_size, \
-                                                                                         size_t lhs_nrows) {           \
-    (void)dim;                                                                                                         \
-    return FaerV0_24_Layout{block_size * lhs_nrows * sizeof(T), 64};                                                   \
-  }                                                                                                                    \
-  void libfaer_v0_23_apply_householder_on_the_right_##SUF(FaerV0_24_MatRef basis, FaerV0_24_MatRef factor, FaerV0_24_Conj conj, \
-                                                          FaerV0_24_MatMut lhs, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) { \
-    (void)conj; (void)par; (void)mem;                                                                                  \
-    householder_seq_entry<T>(basis, factor, transposed(lhs), true);                                                    \
-  }                                                                                                                    \
-  void libfaer_v0_23_apply_householder_transpose_on_the_right_##SUF(FaerV0_24_MatRef basis, FaerV0_24_MatRef factor,   \
-                                                                    FaerV0_24_Conj conj, FaerV0_24_MatMut lhs,         \
-                                                                    FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {       \
-    (void)conj; (void)par; (void)mem;                                                                                  \
-    householder_seq_entry<T>(basis, factor, transposed(lhs), false);                                                   \
-  }                                                                                                                    \
-  /* scratch: apply_block_householder_sequence_[transpose_]on_the_left_in_place_scratch (solve.rs:3-37) */           \
-  FaerV0_24_Layout libfaer_v0_23_qr_solve_lstsq_in_place_scratch_##SUF(size_t nrows, size_t ncols, size_t block_size,  \
-                                                                       size_t rhs_ncols, FaerV0_24_Par par) {          \
-    (void)nrows; (void)ncols; (void)par;                                                                               \
-    return FaerV0_24_Layout{block_size * rhs_ncols * sizeof(T), 64};                                                   \
-  }                                                                                                                    \
-  FaerV0_24_Layout libfaer_v0_23_qr_solve_in_place_scratch_##SUF(size_t dim, size_t block_size, size_t rhs_ncols,      \
-                                                                 FaerV0_24_Par par) {                                  \
-    (void)dim; (void)par;                                                                                              \
-    return FaerV0_24_Layout{block_size * rhs_ncols * sizeof(T), 64};                                                   \
-  }                                                                                                                    \
-  FaerV0_24_Layout libfaer_v0_23_qr_solve_transpose_in_place_scratch_##SUF(size_t dim, size_t block_size,              \
-                                                                           size_t rhs_ncols, FaerV0_24_Par par) {      \
-    (void)dim; (void)par;                                                                                              \
-    return FaerV0_24_Layout{block_size * rhs_ncols * sizeof(T), 64};                                                   \
-  }                                                                                                                    \
-  void libfaer_v0_23_qr_solve_lstsq_in_place_##SUF(FaerV0_24_MatRef Q_basis, FaerV0_24_MatRef Q_coeff, FaerV0_24_MatRef R, \
-                                                   FaerV0_24_Conj A_conj, FaerV0_24_MatMut rhs, FaerV0_24_Par par,     \
-                                                   FaerV0_24_MemAlloc mem) {                                           \
-    (void)A_conj; (void)par; (void)mem;                                                                                \
-    qr_solve_entry<T>(Q_basis, Q_coeff, R, rhs, 0);                                                                    \
-  }                                                                                                                    \
-  void libfaer_v0_23_qr_solve_in_place_##SUF(FaerV0_24_MatRef Q_basis, FaerV0_24_MatRef Q_coeff, FaerV0_24_MatRef R,   \
-                                             FaerV0_24_Conj A_conj, FaerV0_24_MatMut rhs, FaerV0_24_Par par,           \
-                                             FaerV0_24_MemAlloc mem) {                                                 \
-    (void)A_conj; (void)par; (void)mem;                                                                                \
-    qr_solve_entry<T>(Q_basis, Q_coeff, R, rhs, 1);                                                                    \
-  }                                                                                                                    \
-  void libfaer_v0_23_qr_solve_transpose_in_place_##SUF(FaerV0_24_MatRef Q_basis, FaerV0_24_MatRef Q_coeff,             \
-                                                       FaerV0_24_MatRef R, FaerV0_24_Conj A_conj, FaerV0_24_MatMut rhs, \
-                                                       FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {                    \
-    (void)A_conj; (void)par; (void)mem;                                                                                \
-    qr_solve_entry<T>(Q_basis, Q_coeff, R, rhs, 2);                                                                    \
+#define FB_LU_QUERIES_IT(IT, BYTES, SUF, ES)                                                                                    \
+  FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_factor_in_place_scratch_##IT##_##SUF(size_t nrows, size_t ncols, FaerV0_24_Par par, \
+                                                                                     FaerV0_24_PartialPivLuParams params) {    \
+    (void)par; (void)params;                                                                                                    \
+    const size_t size = nrows < ncols ? nrows : ncols; /* StackReq::new::<I>(min(nrows, ncols)) (factor.rs:224-233) */          \
+    return FaerV0_24_Layout{size * (BYTES), (BYTES)};                                                                           \
+  }                                                                                                                             \
+  FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_solve_in_place_scratch_##IT##_##SUF(size_t dim, size_t rhs_ncols, FaerV0_24_Par par) { \
+    (void)par;                                                                                                                  \
+    return FaerV0_24_Layout{dim * rhs_ncols * (ES), 64}; /* permute_rows_in_place_scratch (perm/mod.rs) */                      \
+  }                                                                                                                             \
+  FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_solve_transpose_in_place_scratch_##IT##_##SUF(size_t dim, size_t rhs_ncols,     \
+                                                                                              FaerV0_24_Par par) {              \
+    (void)par;                                                                                                                  \
+    return FaerV0_24_Layout{dim * rhs_ncols * (ES), 64};                                                                        \
   }
-FB_QR_FFI(f64, double)
-FB_QR_FFI(f32, float)
-#undef FB_QR_FFI
+#define FB_LU_QUERIES(SUF, ES)                                                                                                  \
+  FaerV0_24_PartialPivLuParams libfaer_v0_23_PartialPivLuParams_##SUF(void) {                                                   \
+    return FaerV0_24_PartialPivLuParams{16, 64, 128 * 128}; /* lu/partial_pivoting/factor.rs:212-222 */                         \
+  }                                                                                                                             \
+  FB_LU_QUERIES_IT(u32, 4, SUF, ES)                                                                                             \
+  FB_LU_QUERIES_IT(u64, 8, SUF, ES)
+#define FB_LU_FFI_IT(IT, BYTES, SUF, R, CX)                                                                                     \
+  FaerV0_24_PartialPivLuStatus libfaer_v0_23_partial_piv_lu_factor_in_place_##IT##_##SUF(                                       \
+      FaerV0_24_MatMut A, FaerV0_24_SliceMut perm_fwd, FaerV0_24_SliceMut perm_bwd, FaerV0_24_Par par, FaerV0_24_MemAlloc mem,   \
+      FaerV0_24_PartialPivLuParams params) {                                                                                    \
+    (void)par; (void)mem;                                                                                                       \
+    return lu_factor_entry<R, CX>(A, perm_fwd, perm_bwd, params, BYTES);                                                        \
+  }                                                                                                                             \
+  void libfaer_v0_23_partial_piv_lu_solve_in_place_##IT##_##SUF(FaerV0_24_MatRef L, FaerV0_24_MatRef U, FaerV0_24_Conj A_conj,  \
+                                                               FaerV0_24_SliceRef perm_fwd, FaerV0_24_SliceRef perm_bwd,        \
+                                                               FaerV0_24_MatMut rhs, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) { \
+    (void)perm_bwd; (void)par; (void)mem;                                                                                       \
+    lu_solve_entry<R, CX>(L, U, A_conj, perm_fwd, rhs, BYTES, false);                                                           \
+  }                                                                                                                             \
+  void libfaer_v0_23_partial_piv_lu_solve_transpose_in_place_##IT##_##SUF(                                                      \
+      FaerV0_24_MatRef L, FaerV0_24_MatRef U, FaerV0_24_Conj A_conj, FaerV0_24_SliceRef perm_fwd, FaerV0_24_SliceRef perm_bwd,   \
+      FaerV0_24_MatMut rhs, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {                                                        \
+    (void)perm_fwd; (void)par; (void)mem;                                                                                       \
+    lu_solve_entry<R, CX>(L, U, A_conj, perm_bwd, rhs, BYTES, true);                                                            \
+  }
+#define FB_LU_FFI(SUF, R, CX) FB_LU_FFI_IT(u32, 4, SUF, R, CX) FB_LU_FFI_IT(u64, 8, SUF, R, CX)
+FB_LU_QUERIES(f64, sizeof(double))
+FB_LU_QUERIES(f32, sizeof(float))
+FB_LU_QUERIES(c64, 2 * sizeof(double))
+FB_LU_QUERIES(c32, 2 * sizeof(float))
+FB_LU_FFI(f64, double, false)
+FB_LU_FFI(f32, float, false)
+FB_LU_FFI(c64, double, true)
+FB_LU_FFI(c32, float, true)
+#undef FB_LU_QUERIES_IT
+#undef FB_LU_QUERIES
+#undef FB_LU_FFI_IT
+#undef FB_LU_FFI
 
-// ---- complex Householder QR, block-Householder sequences and the QR solves (cplx.cu) ----
-#define FB_QR_CPLX_FFI(SUF, R)                                                                                                  \
+// ---- Householder QR (no pivoting), block-Householder sequences and the QR solves ----
+// scratch: temp_mat_scratch(block_size, ncols) for the factorization, the block-Householder sequence scratch
+// temp_mat_scratch(block_size, rhs_ncols) for the sequences and the solves (solve.rs:3-37)
+#define FB_QR_QUERIES(SUF, ES)                                                                                                  \
   FaerV0_24_QrParams libfaer_v0_23_QrParams_##SUF(void) { return FaerV0_24_QrParams{48 * 48, 192 * 256}; }                      \
   size_t libfaer_v0_23_qr_recommended_block_size_##SUF(size_t nrows, size_t ncols) {                                            \
     return (size_t)qr_recommended_block_size((i64)nrows, (i64)ncols);                                                           \
@@ -970,414 +538,173 @@ FB_QR_FFI(f32, float)
   FaerV0_24_Layout libfaer_v0_23_qr_factor_in_place_scratch_##SUF(size_t nrows, size_t ncols, size_t block_size,                \
                                                                   FaerV0_24_Par par, FaerV0_24_QrParams params) {               \
     (void)nrows; (void)par; (void)params;                                                                                       \
-    return FaerV0_24_Layout{block_size * ncols * 2 * sizeof(R), 64};                                                            \
-  }                                                                                                                             \
-  FaerV0_24_QrStatus libfaer_v0_23_qr_factor_in_place_##SUF(FaerV0_24_MatMut A, FaerV0_24_MatMut Q_coeff, FaerV0_24_Par par,    \
-                                                            FaerV0_24_MemAlloc mem, FaerV0_24_QrParams params) {                \
-    (void)par; (void)mem;                                                                                                       \
-    return qr_entry_cplx<R>(A, Q_coeff, params);                                                                                \
+    return FaerV0_24_Layout{block_size * ncols * (ES), 64};                                                                     \
   }                                                                                                                             \
   FaerV0_24_Layout libfaer_v0_23_apply_householder_on_the_left_scratch_##SUF(size_t dim, size_t block_size, size_t rhs_ncols) { \
     (void)dim;                                                                                                                  \
-    return FaerV0_24_Layout{block_size * rhs_ncols * 2 * sizeof(R), 64};                                                        \
+    return FaerV0_24_Layout{block_size * rhs_ncols * (ES), 64};                                                                 \
   }                                                                                                                             \
   FaerV0_24_Layout libfaer_v0_23_apply_householder_transpose_on_the_left_scratch_##SUF(size_t dim, size_t block_size,           \
                                                                                         size_t rhs_ncols) {                     \
     (void)dim;                                                                                                                  \
-    return FaerV0_24_Layout{block_size * rhs_ncols * 2 * sizeof(R), 64};                                                        \
+    return FaerV0_24_Layout{block_size * rhs_ncols * (ES), 64};                                                                 \
+  }                                                                                                                             \
+  FaerV0_24_Layout libfaer_v0_23_apply_householder_on_the_right_scratch_##SUF(size_t dim, size_t block_size, size_t lhs_nrows) { \
+    (void)dim;                                                                                                                  \
+    return FaerV0_24_Layout{block_size * lhs_nrows * (ES), 64};                                                                 \
+  }                                                                                                                             \
+  FaerV0_24_Layout libfaer_v0_23_apply_householder_transpose_on_the_right_scratch_##SUF(size_t dim, size_t block_size,          \
+                                                                                         size_t lhs_nrows) {                    \
+    (void)dim;                                                                                                                  \
+    return FaerV0_24_Layout{block_size * lhs_nrows * (ES), 64};                                                                 \
+  }                                                                                                                             \
+  FaerV0_24_Layout libfaer_v0_23_qr_solve_lstsq_in_place_scratch_##SUF(size_t nrows, size_t ncols, size_t block_size,           \
+                                                                       size_t rhs_ncols, FaerV0_24_Par par) {                   \
+    (void)nrows; (void)ncols; (void)par;                                                                                        \
+    return FaerV0_24_Layout{block_size * rhs_ncols * (ES), 64};                                                                 \
+  }                                                                                                                             \
+  FaerV0_24_Layout libfaer_v0_23_qr_solve_in_place_scratch_##SUF(size_t dim, size_t block_size, size_t rhs_ncols,               \
+                                                                 FaerV0_24_Par par) {                                           \
+    (void)dim; (void)par;                                                                                                       \
+    return FaerV0_24_Layout{block_size * rhs_ncols * (ES), 64};                                                                 \
+  }                                                                                                                             \
+  FaerV0_24_Layout libfaer_v0_23_qr_solve_transpose_in_place_scratch_##SUF(size_t dim, size_t block_size,                       \
+                                                                           size_t rhs_ncols, FaerV0_24_Par par) {               \
+    (void)dim; (void)par;                                                                                                       \
+    return FaerV0_24_Layout{block_size * rhs_ncols * (ES), 64};                                                                 \
+  }
+#define FB_QR_FFI(SUF, R, CX)                                                                                                   \
+  FaerV0_24_QrStatus libfaer_v0_23_qr_factor_in_place_##SUF(FaerV0_24_MatMut A, FaerV0_24_MatMut Q_coeff, FaerV0_24_Par par,    \
+                                                            FaerV0_24_MemAlloc mem, FaerV0_24_QrParams params) {                \
+    (void)par; (void)mem;                                                                                                       \
+    return qr_factor_entry<R, CX>(A, Q_coeff, params);                                                                          \
   }                                                                                                                             \
   void libfaer_v0_23_apply_householder_on_the_left_##SUF(FaerV0_24_MatRef basis, FaerV0_24_MatRef factor, FaerV0_24_Conj conj,  \
                                                          FaerV0_24_MatMut rhs, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {     \
     (void)par; (void)mem;                                                                                                       \
-    householder_seq_entry_cplx<R>(basis, factor, conj, rhs, false);                                                             \
+    householder_seq_entry<R, CX>(basis, factor, conj, rhs, false);                                                              \
   }                                                                                                                             \
   void libfaer_v0_23_apply_householder_transpose_on_the_left_##SUF(FaerV0_24_MatRef basis, FaerV0_24_MatRef factor,             \
                                                                    FaerV0_24_Conj conj, FaerV0_24_MatMut rhs,                   \
                                                                    FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {                 \
     (void)par; (void)mem;                                                                                                       \
-    householder_seq_entry_cplx<R>(basis, factor, conj, rhs, true);                                                              \
+    householder_seq_entry<R, CX>(basis, factor, conj, rhs, true);                                                               \
   }                                                                                                                             \
   /* on the right = the transposed sequence on the left of the transposed view, and vice versa (householder.rs:813-854) */     \
-  FaerV0_24_Layout libfaer_v0_23_apply_householder_on_the_right_scratch_##SUF(size_t dim, size_t block_size, size_t lhs_nrows) { \
-    (void)dim;                                                                                                                  \
-    return FaerV0_24_Layout{block_size * lhs_nrows * 2 * sizeof(R), 64};                                                        \
-  }                                                                                                                             \
-  FaerV0_24_Layout libfaer_v0_23_apply_householder_transpose_on_the_right_scratch_##SUF(size_t dim, size_t block_size,          \
-                                                                                         size_t lhs_nrows) {                    \
-    (void)dim;                                                                                                                  \
-    return FaerV0_24_Layout{block_size * lhs_nrows * 2 * sizeof(R), 64};                                                        \
-  }                                                                                                                             \
   void libfaer_v0_23_apply_householder_on_the_right_##SUF(FaerV0_24_MatRef basis, FaerV0_24_MatRef factor, FaerV0_24_Conj conj, \
                                                           FaerV0_24_MatMut lhs, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {    \
     (void)par; (void)mem;                                                                                                       \
-    householder_seq_entry_cplx<R>(basis, factor, conj, transposed(lhs), true);                                                  \
+    householder_seq_entry<R, CX>(basis, factor, conj, transposed(lhs), true);                                                   \
   }                                                                                                                             \
   void libfaer_v0_23_apply_householder_transpose_on_the_right_##SUF(FaerV0_24_MatRef basis, FaerV0_24_MatRef factor,            \
                                                                     FaerV0_24_Conj conj, FaerV0_24_MatMut lhs,                  \
                                                                     FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {                \
     (void)par; (void)mem;                                                                                                       \
-    householder_seq_entry_cplx<R>(basis, factor, conj, transposed(lhs), false);                                                 \
-  }                                                                                                                             \
-  FaerV0_24_Layout libfaer_v0_23_qr_solve_lstsq_in_place_scratch_##SUF(size_t nrows, size_t ncols, size_t block_size,           \
-                                                                       size_t rhs_ncols, FaerV0_24_Par par) {                   \
-    (void)nrows; (void)ncols; (void)par;                                                                                        \
-    return FaerV0_24_Layout{block_size * rhs_ncols * 2 * sizeof(R), 64};                                                        \
-  }                                                                                                                             \
-  FaerV0_24_Layout libfaer_v0_23_qr_solve_in_place_scratch_##SUF(size_t dim, size_t block_size, size_t rhs_ncols,               \
-                                                                 FaerV0_24_Par par) {                                           \
-    (void)dim; (void)par;                                                                                                       \
-    return FaerV0_24_Layout{block_size * rhs_ncols * 2 * sizeof(R), 64};                                                        \
-  }                                                                                                                             \
-  FaerV0_24_Layout libfaer_v0_23_qr_solve_transpose_in_place_scratch_##SUF(size_t dim, size_t block_size,                       \
-                                                                           size_t rhs_ncols, FaerV0_24_Par par) {               \
-    (void)dim; (void)par;                                                                                                       \
-    return FaerV0_24_Layout{block_size * rhs_ncols * 2 * sizeof(R), 64};                                                        \
+    householder_seq_entry<R, CX>(basis, factor, conj, transposed(lhs), false);                                                  \
   }                                                                                                                             \
   void libfaer_v0_23_qr_solve_lstsq_in_place_##SUF(FaerV0_24_MatRef Q_basis, FaerV0_24_MatRef Q_coeff, FaerV0_24_MatRef Rm,     \
                                                    FaerV0_24_Conj A_conj, FaerV0_24_MatMut rhs, FaerV0_24_Par par,              \
                                                    FaerV0_24_MemAlloc mem) {                                                    \
     (void)par; (void)mem;                                                                                                       \
-    qr_solve_entry_cplx<R>(Q_basis, Q_coeff, Rm, A_conj, rhs, 0);                                                               \
+    qr_solve_entry<R, CX>(Q_basis, Q_coeff, Rm, A_conj, rhs, 0);                                                                \
   }                                                                                                                             \
   void libfaer_v0_23_qr_solve_in_place_##SUF(FaerV0_24_MatRef Q_basis, FaerV0_24_MatRef Q_coeff, FaerV0_24_MatRef Rm,           \
                                              FaerV0_24_Conj A_conj, FaerV0_24_MatMut rhs, FaerV0_24_Par par,                    \
                                              FaerV0_24_MemAlloc mem) {                                                          \
     (void)par; (void)mem;                                                                                                       \
-    qr_solve_entry_cplx<R>(Q_basis, Q_coeff, Rm, A_conj, rhs, 1);                                                               \
+    qr_solve_entry<R, CX>(Q_basis, Q_coeff, Rm, A_conj, rhs, 1);                                                                \
   }                                                                                                                             \
   void libfaer_v0_23_qr_solve_transpose_in_place_##SUF(FaerV0_24_MatRef Q_basis, FaerV0_24_MatRef Q_coeff,                      \
                                                        FaerV0_24_MatRef Rm, FaerV0_24_Conj A_conj, FaerV0_24_MatMut rhs,        \
                                                        FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {                             \
     (void)par; (void)mem;                                                                                                       \
-    qr_solve_entry_cplx<R>(Q_basis, Q_coeff, Rm, A_conj, rhs, 2);                                                               \
+    qr_solve_entry<R, CX>(Q_basis, Q_coeff, Rm, A_conj, rhs, 2);                                                                \
   }
-FB_QR_CPLX_FFI(c64, double)
-FB_QR_CPLX_FFI(c32, float)
-#undef FB_QR_CPLX_FFI
+FB_QR_QUERIES(f64, sizeof(double))
+FB_QR_QUERIES(f32, sizeof(float))
+FB_QR_QUERIES(c64, 2 * sizeof(double))
+FB_QR_QUERIES(c32, 2 * sizeof(float))
+FB_QR_FFI(f64, double, false)
+FB_QR_FFI(f32, float, false)
+FB_QR_FFI(c64, double, true)
+FB_QR_FFI(c32, float, true)
+#undef FB_QR_QUERIES
+#undef FB_QR_FFI
 
-// ---- solves on top of the factors ----
-FaerV0_24_Layout libfaer_v0_23_llt_solve_in_place_scratch_f64(size_t dim, size_t rhs_ncols, FaerV0_24_Par par) {
-  (void)dim; (void)rhs_ncols; (void)par;
-  return FaerV0_24_Layout{0, 1};  // reference: StackReq::EMPTY (llt/solve.rs:3-10)
-}
-void libfaer_v0_23_llt_solve_in_place_f64(FaerV0_24_MatRef L, FaerV0_24_Conj A_conj, FaerV0_24_MatMut rhs, FaerV0_24_Par par,
-                                          FaerV0_24_MemAlloc mem) {
-  (void)A_conj; (void)par; (void)mem;
-  FB_ENTRY();
-  cudaStream_t st = current_stream();
-  FB_ASSERT(L.nrows == L.ncols && rhs.nrows == L.nrows, "LLT solve shape mismatch");
-  Mat l(L, st);
-  Mat r(rhs, true, st);
-  llt_solve_in_place_f64(st, l.s.view<const double>(), r.s.view<double>());
-  finish_all(st, {&l.s, &r.s});
-}
-
-// transpose = false: perm is perm_fwd (solve.rs:21-54); transpose = true: perm is perm_bwd (solve.rs:55-86)
-static void lu_solve_entry(FaerV0_24_MatRef L, FaerV0_24_MatRef U, FaerV0_24_SliceRef perm_slice, FaerV0_24_MatMut rhs,
-                           int idx_bytes, bool transpose = false) {
-  FB_ENTRY();
-  cudaStream_t st = current_stream();
-  const size_t n = L.nrows;
-  FB_ASSERT(L.ncols == n && U.nrows == n && U.ncols == n && rhs.nrows == n, "LU solve shape mismatch");
-  std::vector<long long> perm = read_perm(perm_slice.ptr, n, idx_bytes);  // length from L.nrows (see lu_entry note)
-  for (size_t i = 0; i < n; ++i) FB_ASSERT(perm[i] >= 0 && (size_t)perm[i] < n, "invalid permutation entry");
-  Mat l(L, st), u(U, st);
-  Mat r(rhs, true, st);
-  if (transpose)
-    lu_solve_transpose_in_place_f64(st, l.s.view<const double>(), u.s.view<const double>(), perm.data(), r.s.view<double>());
-  else
-    lu_solve_in_place_f64(st, l.s.view<const double>(), u.s.view<const double>(), perm.data(), r.s.view<double>());
-  finish_all(st, {&l.s, &u.s, &r.s});
-}
-FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_solve_in_place_scratch_u32_f64(size_t dim, size_t rhs_ncols, FaerV0_24_Par par) {
-  (void)par;
-  return FaerV0_24_Layout{dim * rhs_ncols * sizeof(double), 64};  // permute_rows_in_place_scratch (perm/mod.rs)
-}
-FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_solve_in_place_scratch_u64_f64(size_t dim, size_t rhs_ncols, FaerV0_24_Par par) {
-  (void)par;
-  return FaerV0_24_Layout{dim * rhs_ncols * sizeof(double), 64};
-}
-void libfaer_v0_23_partial_piv_lu_solve_in_place_u32_f64(FaerV0_24_MatRef L, FaerV0_24_MatRef U, FaerV0_24_Conj A_conj,
-                                                         FaerV0_24_SliceRef perm_fwd, FaerV0_24_SliceRef perm_bwd,
-                                                         FaerV0_24_MatMut rhs, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {
-  (void)A_conj; (void)perm_bwd; (void)par; (void)mem;
-  lu_solve_entry(L, U, perm_fwd, rhs, 4);
-}
-void libfaer_v0_23_partial_piv_lu_solve_in_place_u64_f64(FaerV0_24_MatRef L, FaerV0_24_MatRef U, FaerV0_24_Conj A_conj,
-                                                         FaerV0_24_SliceRef perm_fwd, FaerV0_24_SliceRef perm_bwd,
-                                                         FaerV0_24_MatMut rhs, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {
-  (void)A_conj; (void)perm_bwd; (void)par; (void)mem;
-  lu_solve_entry(L, U, perm_fwd, rhs, 8);
-}
-FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_solve_transpose_in_place_scratch_u32_f64(size_t dim, size_t rhs_ncols, FaerV0_24_Par par) {
-  (void)par;
-  return FaerV0_24_Layout{dim * rhs_ncols * sizeof(double), 64};
-}
-FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_solve_transpose_in_place_scratch_u64_f64(size_t dim, size_t rhs_ncols, FaerV0_24_Par par) {
-  (void)par;
-  return FaerV0_24_Layout{dim * rhs_ncols * sizeof(double), 64};
-}
-void libfaer_v0_23_partial_piv_lu_solve_transpose_in_place_u32_f64(FaerV0_24_MatRef L, FaerV0_24_MatRef U, FaerV0_24_Conj A_conj,
-                                                                   FaerV0_24_SliceRef perm_fwd, FaerV0_24_SliceRef perm_bwd,
-                                                                   FaerV0_24_MatMut rhs, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {
-  (void)A_conj; (void)perm_fwd; (void)par; (void)mem;
-  lu_solve_entry(L, U, perm_bwd, rhs, 4, true);
-}
-void libfaer_v0_23_partial_piv_lu_solve_transpose_in_place_u64_f64(FaerV0_24_MatRef L, FaerV0_24_MatRef U, FaerV0_24_Conj A_conj,
-                                                                   FaerV0_24_SliceRef perm_fwd, FaerV0_24_SliceRef perm_bwd,
-                                                                   FaerV0_24_MatMut rhs, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {
-  (void)A_conj; (void)perm_fwd; (void)par; (void)mem;
-  lu_solve_entry(L, U, perm_bwd, rhs, 8, true);
-}
-
-// f32 LU solves (lu/partial_pivoting/solve.rs:21-86) on the native f32 triangular solves
-static void lu_solve_entry_f32(FaerV0_24_MatRef L, FaerV0_24_MatRef U, FaerV0_24_SliceRef perm_slice, FaerV0_24_MatMut rhs,
-                               int idx_bytes, bool transpose) {
-  FB_ENTRY();
-  cudaStream_t st = current_stream();
-  const size_t n = L.nrows;
-  FB_ASSERT(L.ncols == n && U.nrows == n && U.ncols == n && rhs.nrows == n, "LU solve shape mismatch");
-  std::vector<long long> perm = read_perm(perm_slice.ptr, n, idx_bytes);
-  for (size_t i = 0; i < n; ++i) FB_ASSERT(perm[i] >= 0 && (size_t)perm[i] < n, "invalid permutation entry");
-  StagedMat l(L.ptr, (i64)L.nrows, (i64)L.ncols, (i64)L.row_stride, (i64)L.col_stride, 4, true, false, st);
-  StagedMat u(U.ptr, (i64)U.nrows, (i64)U.ncols, (i64)U.row_stride, (i64)U.col_stride, 4, true, false, st);
-  StagedMat r(rhs.ptr, (i64)rhs.nrows, (i64)rhs.ncols, (i64)rhs.row_stride, (i64)rhs.col_stride, 4, true, true, st);
-  VCF lv = l.view<const float>(), uv = u.view<const float>();
-  VF rv = r.view<float>();
-  const i64 k = rv.ncols;
-  auto permute = [&]() {  // rhs[i, :] <- rhs[perm[i], :]
-    if (n == 0 || k == 0) return;
-    FB_ASSERT(k < 65536, "too many right-hand sides for one permutation launch");
-    long long* d_perm = (long long*)ws_alloc(n * 8);
-    float* tmp = (float*)ws_alloc(n * (size_t)k * 4);
-    FB_CUDA_CHECK(cudaMemcpyAsync(d_perm, perm.data(), n * 8, cudaMemcpyHostToDevice, st));
-    ffi_gather_rows_f32_kernel<<<dim3((unsigned)((n + 255) / 256), (unsigned)k), 256, 0, st>>>(tmp, rv.ptr, rv.rs, rv.cs, (i64)n, d_perm);
-    note_launch();
-    ffi_cast<float, float>(st, rv.ptr, rv.rs, rv.cs, tmp, 1, (i64)n, (i64)n, k);
-    FB_CUDA_CHECK(cudaStreamSynchronize(st));
-    ws_free(tmp);
-    ws_free(d_perm);
-  };
-  if (!transpose) {
-    permute();
-    solve_lower_triangular_in_place_f32(st, lv, true, rv);
-    solve_upper_triangular_in_place_f32(st, uv, false, rv);
-  } else {
-    solve_lower_triangular_in_place_f32(st, uv.t(), false, rv);
-    solve_upper_triangular_in_place_f32(st, lv.t(), true, rv);
-    permute();
-  }
-  finish_all(st, {&l, &u, &r});
-}
-#define FB_LU_SOLVE_F32(IT, BYTES)                                                                                              \
-  FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_solve_in_place_scratch_##IT##_f32(size_t dim, size_t rhs_ncols, FaerV0_24_Par par) { \
-    (void)par;                                                                                                                  \
-    return FaerV0_24_Layout{dim * rhs_ncols * sizeof(float), 64};                                                               \
+// ---- SVD / self-adjoint EVD for real T (svd.cu / evd.cu: values by bisection; svd_vectors.cu + tridiag_dc.cu: with vectors) ----
+#define FB_SVD_EVD_FFI(SUF, T)                                                                                                  \
+  FaerV0_24_SvdStatus libfaer_v0_23_svd_##SUF(FaerV0_24_MatRef A, FaerV0_24_MatMut U, FaerV0_24_VecMut S, FaerV0_24_MatMut V,   \
+                                              FaerV0_24_Par par, FaerV0_24_MemAlloc mem, FaerV0_24_SvdParams params) {          \
+    (void)par; (void)mem;                                                                                                       \
+    return svd_entry<T>(A, U, S, V, params.qr_ratio_threshold);                                                                 \
   }                                                                                                                             \
-  void libfaer_v0_23_partial_piv_lu_solve_in_place_##IT##_f32(FaerV0_24_MatRef L, FaerV0_24_MatRef U, FaerV0_24_Conj A_conj,    \
-                                                             FaerV0_24_SliceRef perm_fwd, FaerV0_24_SliceRef perm_bwd,          \
-                                                             FaerV0_24_MatMut rhs, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) { \
-    (void)A_conj; (void)perm_bwd; (void)par; (void)mem;                                                                         \
-    lu_solve_entry_f32(L, U, perm_fwd, rhs, BYTES, false);                                                                      \
-  }                                                                                                                             \
-  FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_solve_transpose_in_place_scratch_##IT##_f32(size_t dim, size_t rhs_ncols,       \
-                                                                                            FaerV0_24_Par par) {                \
-    (void)par;                                                                                                                  \
-    return FaerV0_24_Layout{dim * rhs_ncols * sizeof(float), 64};                                                               \
-  }                                                                                                                             \
-  void libfaer_v0_23_partial_piv_lu_solve_transpose_in_place_##IT##_f32(                                                        \
-      FaerV0_24_MatRef L, FaerV0_24_MatRef U, FaerV0_24_Conj A_conj, FaerV0_24_SliceRef perm_fwd, FaerV0_24_SliceRef perm_bwd,   \
-      FaerV0_24_MatMut rhs, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {                                                        \
-    (void)A_conj; (void)perm_fwd; (void)par; (void)mem;                                                                         \
-    lu_solve_entry_f32(L, U, perm_bwd, rhs, BYTES, true);                                                                       \
-  }
-FB_LU_SOLVE_F32(u32, 4)
-FB_LU_SOLVE_F32(u64, 8)
-#undef FB_LU_SOLVE_F32
-
-// ---- c64 / c32 partial-pivoting LU (cplx.cu) ----
-FaerV0_24_PartialPivLuParams libfaer_v0_23_PartialPivLuParams_c64(void) { return libfaer_v0_23_PartialPivLuParams_f64(); }
-FaerV0_24_PartialPivLuParams libfaer_v0_23_PartialPivLuParams_c32(void) { return libfaer_v0_23_PartialPivLuParams_f64(); }
-#define FB_LU_CPLX(IT, BYTES, SUF, R)                                                                                           \
-  FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_factor_in_place_scratch_##IT##_##SUF(size_t nrows, size_t ncols, FaerV0_24_Par par, \
-                                                                                     FaerV0_24_PartialPivLuParams params) {    \
-    (void)par; (void)params;                                                                                                    \
-    return lu_scratch(nrows, ncols, BYTES);                                                                                     \
-  }                                                                                                                             \
-  FaerV0_24_PartialPivLuStatus libfaer_v0_23_partial_piv_lu_factor_in_place_##IT##_##SUF(                                       \
-      FaerV0_24_MatMut A, FaerV0_24_SliceMut perm_fwd, FaerV0_24_SliceMut perm_bwd, FaerV0_24_Par par, FaerV0_24_MemAlloc mem,   \
-      FaerV0_24_PartialPivLuParams params) {                                                                                    \
+  FaerV0_24_EvdStatus libfaer_v0_23_self_adjoint_evd_##SUF(FaerV0_24_MatRef A, FaerV0_24_MatMut U, FaerV0_24_VecMut S,          \
+                                                           FaerV0_24_Par par, FaerV0_24_MemAlloc mem,                           \
+                                                           FaerV0_24_SelfAdjointEvdParams params) {                             \
     (void)par; (void)mem; (void)params;                                                                                         \
-    return lu_entry_cplx<R>(A, perm_fwd, perm_bwd, BYTES);                                                                      \
-  }                                                                                                                             \
-  FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_solve_in_place_scratch_##IT##_##SUF(size_t dim, size_t rhs_ncols, FaerV0_24_Par par) { \
-    (void)par;                                                                                                                  \
-    return FaerV0_24_Layout{dim * rhs_ncols * 2 * sizeof(R), 64};                                                               \
-  }                                                                                                                             \
-  void libfaer_v0_23_partial_piv_lu_solve_in_place_##IT##_##SUF(FaerV0_24_MatRef L, FaerV0_24_MatRef U, FaerV0_24_Conj A_conj,  \
-                                                               FaerV0_24_SliceRef perm_fwd, FaerV0_24_SliceRef perm_bwd,        \
-                                                               FaerV0_24_MatMut rhs, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) { \
-    (void)perm_bwd; (void)par; (void)mem;                                                                                       \
-    lu_solve_entry_cplx<R>(L, U, A_conj, perm_fwd, rhs, BYTES);                                                                 \
-  }                                                                                                                             \
-  FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_solve_transpose_in_place_scratch_##IT##_##SUF(size_t dim, size_t rhs_ncols,     \
-                                                                                              FaerV0_24_Par par) {              \
-    (void)par;                                                                                                                  \
-    return FaerV0_24_Layout{dim * rhs_ncols * 2 * sizeof(R), 64};                                                               \
-  }                                                                                                                             \
-  void libfaer_v0_23_partial_piv_lu_solve_transpose_in_place_##IT##_##SUF(                                                      \
-      FaerV0_24_MatRef L, FaerV0_24_MatRef U, FaerV0_24_Conj A_conj, FaerV0_24_SliceRef perm_fwd, FaerV0_24_SliceRef perm_bwd,   \
-      FaerV0_24_MatMut rhs, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {                                                        \
-    (void)perm_fwd; (void)par; (void)mem;                                                                                       \
-    lu_solve_entry_cplx<R>(L, U, A_conj, perm_bwd, rhs, BYTES, true);                                                           \
+    return self_adjoint_evd_entry<T>(A, U, S);                                                                                  \
   }
-FB_LU_CPLX(u32, 4, c64, double)
-FB_LU_CPLX(u64, 8, c64, double)
-FB_LU_CPLX(u32, 4, c32, float)
-FB_LU_CPLX(u64, 8, c32, float)
-#undef FB_LU_CPLX
+FB_SVD_EVD_FFI(f64, double)
+FB_SVD_EVD_FFI(f32, float)
+#undef FB_SVD_EVD_FFI
 
-// ---- SVD (svd.cu: values by bisection; svd_vectors.cu: with U / V) ----
-#define FB_SVD_FFI(SUF, T)                                                                                             \
-  FaerV0_24_BidiagParams libfaer_v0_23_BidiagParams_##SUF(void) { return FaerV0_24_BidiagParams{192 * 256}; }          \
-  FaerV0_24_SvdParams libfaer_v0_23_SvdParams_##SUF(void) {                                                            \
-    /* svd/mod.rs:49-58: recursion_threshold 128, qr_ratio_threshold 11/6 */                                          \
-    return FaerV0_24_SvdParams{FaerV0_24_BidiagParams{192 * 256}, FaerV0_24_QrParams{48 * 48, 192 * 256}, 128, 11.0 / 6.0}; \
-  }                                                                                                                    \
-  FaerV0_24_Layout libfaer_v0_23_svd_scratch_##SUF(size_t nrows, size_t ncols, FaerV0_24_ComputeSvdVectors compute_U,  \
-                                                   FaerV0_24_ComputeSvdVectors compute_V, FaerV0_24_Par par,           \
-                                                   FaerV0_24_SvdParams params) {                                       \
-    (void)compute_U; (void)compute_V; (void)par; (void)params;                                                         \
-    /* the GPU path keeps its workspace (a copy of A) in the device pool; reported so that callers size like faer */   \
-    return FaerV0_24_Layout{nrows * ncols * sizeof(T), 64};                                                            \
-  }                                                                                                                    \
-  FaerV0_24_SvdStatus libfaer_v0_23_svd_##SUF(FaerV0_24_MatRef A, FaerV0_24_MatMut U, FaerV0_24_VecMut S, FaerV0_24_MatMut V, \
-                                              FaerV0_24_Par par, FaerV0_24_MemAlloc mem, FaerV0_24_SvdParams params) { \
-    (void)par; (void)mem;                                                                                              \
-    return svd_entry<T>(A, U, S, V, params.qr_ratio_threshold);                                                        \
-  }
-FB_SVD_FFI(f64, double)
-FB_SVD_FFI(f32, float)
-#undef FB_SVD_FFI
-
-// ---- self-adjoint EVD (evd.cu: values by bisection; svd_vectors.cu + tridiag_dc.cu: with eigenvectors) ----
-#define FB_EVD_FFI(SUF, T)                                                                                             \
-  FaerV0_24_TridiagParams libfaer_v0_23_TridiagParams_##SUF(void) { return FaerV0_24_TridiagParams{192 * 256}; }       \
-  FaerV0_24_SelfAdjointEvdParams libfaer_v0_23_SelfAdjointEvdParams_##SUF(void) {                                      \
-    return FaerV0_24_SelfAdjointEvdParams{FaerV0_24_TridiagParams{192 * 256}, 128}; /* evd/mod.rs:82-90 */             \
-  }                                                                                                                    \
-  FaerV0_24_Layout libfaer_v0_23_self_adjoint_evd_scratch_##SUF(size_t dim, FaerV0_24_ComputeEigenvectors compute_U,   \
-                                                                FaerV0_24_Par par, FaerV0_24_SelfAdjointEvdParams params) { \
-    (void)compute_U; (void)par; (void)params;                                                                          \
-    return FaerV0_24_Layout{dim * dim * sizeof(T), 64}; /* the copy of A (kept in the device pool here) */             \
-  }                                                                                                                    \
-  FaerV0_24_EvdStatus libfaer_v0_23_self_adjoint_evd_##SUF(FaerV0_24_MatRef A, FaerV0_24_MatMut U, FaerV0_24_VecMut S, \
-                                                           FaerV0_24_Par par, FaerV0_24_MemAlloc mem,                  \
-                                                           FaerV0_24_SelfAdjointEvdParams params) {                    \
-    (void)par; (void)mem; (void)params;                                                                                \
-    return self_adjoint_evd_entry<T>(A, U, S);                                                                         \
-  }
-FB_EVD_FFI(f64, double)
-FB_EVD_FFI(f32, float)
-#undef FB_EVD_FFI
-
-// ---- reconstruct / inverse on the factors (reconstruct.cu; f64, qr_reconstruct also f32) ----
-FaerV0_24_Layout libfaer_v0_23_llt_reconstruct_scratch_f64(size_t dim, FaerV0_24_Par par) {
-  (void)dim; (void)par;
-  return FaerV0_24_Layout{0, 1};  // StackReq::EMPTY (llt/reconstruct.rs:3-6)
-}
+// ---- reconstruct / inverse on the factors, f64 (reconstruct.cu; qr_reconstruct also f32; the queries: ffi_types.cu) ----
 void libfaer_v0_23_llt_reconstruct_f64(FaerV0_24_MatMut A, FaerV0_24_MatRef L, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {
   (void)par; (void)mem;
   FB_ENTRY();
   cudaStream_t st = current_stream();
-  Mat a(A, true, st);  // only the lower triangle is written: the rest of A must survive the round trip
-  Mat l(L, st);
-  llt_reconstruct_f64(st, a.s.view<double>(), l.s.view<const double>());
-  finish_all(st, {&a.s, &l.s});
-}
-FaerV0_24_Layout libfaer_v0_23_llt_inverse_scratch_f64(size_t dim, FaerV0_24_Par par) {
-  (void)par;
-  return FaerV0_24_Layout{dim * dim * sizeof(double), 64};  // temp_mat_scratch(dim, dim) (llt/inverse.rs:3-8)
+  // only the lower triangle is written: the rest of A must survive the round trip
+  StagedMat a = stage(A, sizeof(double), true, st), l = stage(L, sizeof(double), st);
+  llt_reconstruct_f64(st, a.view<double>(), l.view<const double>());
+  finish_all(st, {&a, &l});
 }
 void libfaer_v0_23_llt_inverse_f64(FaerV0_24_MatMut A_inv, FaerV0_24_MatRef L, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {
   (void)par; (void)mem;
   FB_ENTRY();
   cudaStream_t st = current_stream();
-  Mat a(A_inv, true, st);
-  Mat l(L, st);
-  llt_inverse_f64(st, a.s.view<double>(), l.s.view<const double>());
-  finish_all(st, {&a.s, &l.s});
+  StagedMat a = stage(A_inv, sizeof(double), true, st), l = stage(L, sizeof(double), st);
+  llt_inverse_f64(st, a.view<double>(), l.view<const double>());
+  finish_all(st, {&a, &l});
 }
-static void lu_recon_entry(FaerV0_24_MatMut A, FaerV0_24_MatRef L, FaerV0_24_MatRef U, FaerV0_24_SliceRef perm, int idx_bytes,
-                           bool inverse) {
-  FB_ENTRY();
-  cudaStream_t st = current_stream();
-  const size_t m = L.nrows;
-  std::vector<long long> p = read_perm(perm.ptr, m, idx_bytes);
-  for (size_t i = 0; i < m; ++i) FB_ASSERT(p[i] >= 0 && (size_t)p[i] < m, "invalid permutation entry");
-  Mat a(A, false, st);
-  Mat l(L, st), u(U, st);
-  if (inverse) lu_inverse_f64(st, a.s.view<double>(), l.s.view<const double>(), u.s.view<const double>(), p.data());
-  else lu_reconstruct_f64(st, a.s.view<double>(), l.s.view<const double>(), u.s.view<const double>(), p.data());
-  finish_all(st, {&a.s, &l.s, &u.s});
-}
-#define FB_LU_RECON_FFI(IT, BYTES)                                                                                     \
-  FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_reconstruct_scratch_##IT##_f64(size_t nrows, size_t ncols, FaerV0_24_Par par) { \
-    (void)par;                                                                                                         \
-    return FaerV0_24_Layout{nrows * ncols * sizeof(double), 64};                                                       \
-  }                                                                                                                    \
-  void libfaer_v0_23_partial_piv_lu_reconstruct_##IT##_f64(FaerV0_24_MatMut A, FaerV0_24_MatRef L, FaerV0_24_MatRef U, \
-                                                           FaerV0_24_SliceRef perm_fwd, FaerV0_24_SliceRef perm_bwd,   \
-                                                           FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {                \
-    (void)perm_fwd; (void)par; (void)mem;                                                                              \
-    lu_recon_entry(A, L, U, perm_bwd, BYTES, false);                                                                   \
-  }                                                                                                                    \
-  FaerV0_24_Layout libfaer_v0_23_partial_piv_lu_inverse_scratch_##IT##_f64(size_t dim, FaerV0_24_Par par) {            \
-    (void)par;                                                                                                         \
-    return FaerV0_24_Layout{dim * dim * sizeof(double), 64};                                                           \
-  }                                                                                                                    \
-  void libfaer_v0_23_partial_piv_lu_inverse_##IT##_f64(FaerV0_24_MatMut A, FaerV0_24_MatRef L, FaerV0_24_MatRef U,     \
-                                                       FaerV0_24_SliceRef perm_fwd, FaerV0_24_SliceRef perm_bwd,       \
-                                                       FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {                    \
-    (void)perm_bwd; (void)par; (void)mem;                                                                              \
-    lu_recon_entry(A, L, U, perm_fwd, BYTES, true);                                                                    \
+#define FB_LU_RECON_FFI(IT, BYTES)                                                                                              \
+  void libfaer_v0_23_partial_piv_lu_reconstruct_##IT##_f64(FaerV0_24_MatMut A, FaerV0_24_MatRef L, FaerV0_24_MatRef U,          \
+                                                           FaerV0_24_SliceRef perm_fwd, FaerV0_24_SliceRef perm_bwd,            \
+                                                           FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {                         \
+    (void)perm_fwd; (void)par; (void)mem;                                                                                       \
+    lu_recon_entry(A, L, U, perm_bwd, BYTES, false);                                                                            \
+  }                                                                                                                             \
+  void libfaer_v0_23_partial_piv_lu_inverse_##IT##_f64(FaerV0_24_MatMut A, FaerV0_24_MatRef L, FaerV0_24_MatRef U,              \
+                                                       FaerV0_24_SliceRef perm_fwd, FaerV0_24_SliceRef perm_bwd,                \
+                                                       FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {                             \
+    (void)perm_bwd; (void)par; (void)mem;                                                                                       \
+    lu_recon_entry(A, L, U, perm_fwd, BYTES, true);                                                                             \
   }
 FB_LU_RECON_FFI(u32, 4)
 FB_LU_RECON_FFI(u64, 8)
 #undef FB_LU_RECON_FFI
-#define FB_QR_RECON_FFI(SUF, T)                                                                                        \
-  FaerV0_24_Layout libfaer_v0_23_qr_reconstruct_scratch_##SUF(size_t nrows, size_t ncols, size_t block_size, FaerV0_24_Par par) { \
-    (void)nrows; (void)par;                                                                                            \
-    return FaerV0_24_Layout{block_size * ncols * sizeof(T), 64};                                                       \
-  }                                                                                                                    \
-  void libfaer_v0_23_qr_reconstruct_##SUF(FaerV0_24_MatMut A, FaerV0_24_MatRef Q_basis, FaerV0_24_MatRef Q_coeff,      \
-                                          FaerV0_24_MatRef R, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {             \
-    (void)par; (void)mem;                                                                                              \
-    FB_ENTRY();                                                                                                        \
-    cudaStream_t st = current_stream();                                                                                \
-    StagedMat a(A.ptr, (i64)A.nrows, (i64)A.ncols, (i64)A.row_stride, (i64)A.col_stride, sizeof(T), false, true, st);  \
-    StagedMat b(Q_basis.ptr, (i64)Q_basis.nrows, (i64)Q_basis.ncols, (i64)Q_basis.row_stride, (i64)Q_basis.col_stride, sizeof(T), true, false, st); \
-    StagedMat f(Q_coeff.ptr, (i64)Q_coeff.nrows, (i64)Q_coeff.ncols, (i64)Q_coeff.row_stride, (i64)Q_coeff.col_stride, sizeof(T), true, false, st); \
-    StagedMat r(R.ptr, (i64)R.nrows, (i64)R.ncols, (i64)R.row_stride, (i64)R.col_stride, sizeof(T), true, false, st);  \
-    qr_reconstruct<T>(st, a.view<T>(), b.view<const T>(), f.view<const T>(), r.view<const T>());                       \
-    finish_all(st, {&a, &b, &f, &r});                                                                                  \
+#define FB_QR_RECON_FFI(SUF, T)                                                                                                 \
+  void libfaer_v0_23_qr_reconstruct_##SUF(FaerV0_24_MatMut A, FaerV0_24_MatRef Q_basis, FaerV0_24_MatRef Q_coeff,               \
+                                          FaerV0_24_MatRef R, FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {                      \
+    (void)par; (void)mem;                                                                                                       \
+    FB_ENTRY();                                                                                                                 \
+    cudaStream_t st = current_stream();                                                                                         \
+    StagedMat a = stage(A, sizeof(T), false, st), b = stage(Q_basis, sizeof(T), st), f = stage(Q_coeff, sizeof(T), st),         \
+              r = stage(R, sizeof(T), st);                                                                                      \
+    qr_reconstruct<T>(st, a.view<T>(), b.view<const T>(), f.view<const T>(), r.view<const T>());                                \
+    finish_all(st, {&a, &b, &f, &r});                                                                                           \
   }
 FB_QR_RECON_FFI(f64, double)
 FB_QR_RECON_FFI(f32, float)
 #undef FB_QR_RECON_FFI
-FaerV0_24_Layout libfaer_v0_23_qr_inverse_scratch_f64(size_t dim, size_t block_size, FaerV0_24_Par par) {
-  (void)par;
-  return FaerV0_24_Layout{block_size * dim * sizeof(double), 64};
-}
 void libfaer_v0_23_qr_inverse_f64(FaerV0_24_MatMut A, FaerV0_24_MatRef Q_basis, FaerV0_24_MatRef Q_coeff, FaerV0_24_MatRef R,
                                   FaerV0_24_Par par, FaerV0_24_MemAlloc mem) {
   (void)par; (void)mem;
   FB_ENTRY();
   cudaStream_t st = current_stream();
-  Mat a(A, false, st);
-  Mat b(Q_basis, st), f(Q_coeff, st), r(R, st);
-  qr_inverse_f64(st, a.s.view<double>(), b.s.view<const double>(), f.s.view<const double>(), r.s.view<const double>());
-  finish_all(st, {&a.s, &b.s, &f.s, &r.s});
+  StagedMat a = stage(A, sizeof(double), false, st), b = stage(Q_basis, sizeof(double), st), f = stage(Q_coeff, sizeof(double), st),
+            r = stage(R, sizeof(double), st);
+  qr_inverse_f64(st, a.view<double>(), b.view<const double>(), f.view<const double>(), r.view<const double>());
+  finish_all(st, {&a, &b, &f, &r});
 }
 
 // ---- global par / alloc ----
@@ -1429,23 +756,10 @@ int faer_b200_dist_init(int rank, int nranks, const void* id128) {
 void faer_b200_dist_finalize(void) { std::lock_guard<std::recursive_mutex> lock(entry_mutex()); dist_finalize(); }
 FaerV0_24_LltStatus faer_b200_dist_llt_factor_in_place_f64(void* A_local, size_t ld, size_t n, size_t nb,
                                                            FaerV0_24_LltRegularization regularization, int lookahead) {
-  double delta = 0.0, eps = 0.0;
-  if (regularization.dynamic_regularization_delta)
-    delta = read_scalar_f64((const FaerV0_24_Scalar*)regularization.dynamic_regularization_delta);
-  if (regularization.dynamic_regularization_epsilon)
-    eps = read_scalar_f64((const FaerV0_24_Scalar*)regularization.dynamic_regularization_epsilon);
+  double delta, eps;
+  read_regularization(regularization, delta, eps);
   FB_ASSERT(n == 0 || is_device_pointer(A_local), "distributed entry points take device-resident local matrices");
-  LltResult r = dist_llt_f64((double*)A_local, (i64)ld, (i64)n, (i64)nb, delta, eps, lookahead);
-  FaerV0_24_LltStatus out;
-  memset(&out, 0, sizeof(out));
-  if (r.ok) {
-    out.tag = FaerV0_24_LltStatus_Ok;
-    out.ok.dynamic_regularization_count = r.dynamic_regularization_count;
-  } else {
-    out.tag = FaerV0_24_LltStatus_NonPositivePivot;
-    out.non_positive_pivot.index = r.non_positive_pivot_index;
-  }
-  return out;
+  return llt_status(dist_llt_f64((double*)A_local, (i64)ld, (i64)n, (i64)nb, delta, eps, lookahead));
 }
 
 size_t faer_b200_dist_partial_piv_lu_factor_in_place_f64(void* A_local, size_t ld, size_t n, size_t nb, long long* perm_fwd,
@@ -1478,9 +792,9 @@ void faer_b200_spicy_matmul_f64(FaerV0_24_MatMut C, FaerV0_24_Block C_block, con
     for (size_t i = 0; i < nrow_idx; ++i) FB_ASSERT(row_idx[i] < C.nrows, "spicy_matmul: row index out of range");
   if (col_idx && !is_device_pointer(col_idx))
     for (size_t j = 0; j < ncol_idx; ++j) FB_ASSERT(col_idx[j] < C.ncols, "spicy_matmul: column index out of range");
-  const double a = read_scalar_f64(alpha);
-  Mat c(C, true, st);  // scattered destinations keep the untouched entries: always stage the old contents
-  Mat lhs(A, st), rhs(B, st);
+  const double a = read_real<double>(alpha);
+  // scattered destinations keep the untouched entries: always stage the old contents
+  StagedMat c = stage(C, sizeof(double), true, st), lhs = stage(A, sizeof(double), st), rhs = stage(B, sizeof(double), st);
   // indices and diagonal: device copies of host arrays
   auto to_dev = [&](const void* p, size_t bytes) -> void* {
     if (!p || bytes == 0) return nullptr;
@@ -1492,9 +806,9 @@ void faer_b200_spicy_matmul_f64(FaerV0_24_MatMut C, FaerV0_24_Block C_block, con
   void* dri = to_dev(row_idx, nrow_idx * 8);
   void* dci = to_dev(col_idx, ncol_idx * 8);
   void* dd = to_dev(D, (size_t)A.ncols * 8);
-  spicy_matmul_f64(st, c.s.view<double>(), (int)C_block, (const long long*)dri, (const long long*)dci,
-                   accum == FaerV0_24_Accum_Add ? 1 : 0, lhs.s.view<const double>(), rhs.s.view<const double>(), (const double*)dd, 1, a);
-  finish_all(st, {&c.s, &lhs.s, &rhs.s});
+  spicy_matmul_f64(st, c.view<double>(), (int)C_block, (const long long*)dri, (const long long*)dci,
+                   accum == FaerV0_24_Accum_Add ? 1 : 0, lhs.view<const double>(), rhs.view<const double>(), (const double*)dd, 1, a);
+  finish_all(st, {&c, &lhs, &rhs});
   if (dri && dri != (void*)row_idx) ws_free(dri);
   if (dci && dci != (void*)col_idx) ws_free(dci);
   if (dd && dd != (void*)D) ws_free(dd);
@@ -1519,9 +833,9 @@ void faer_b200_gemm(int dtype, int itype, int instr_set, size_t m, size_t n, siz
   if (plain && dtype != FaerB200_GemmDType_F64) {
     FaerV0_24_MatMut C{dst, m, n, dst_rs, dst_cs};
     const FaerV0_24_Scalar* a = (const FaerV0_24_Scalar*)alpha;
-    if (dtype == FaerB200_GemmDType_F32) matmul_f32_impl(C, block, acc, A, 0, B, 0, a);
-    else if (dtype == FaerB200_GemmDType_C64) matmul_c64_impl(C, block, acc, A, 0, B, 0, a, conj_lhs, conj_rhs);
-    else matmul_c32_impl(C, block, acc, A, 0, B, 0, a, conj_lhs, conj_rhs);
+    if (dtype == FaerB200_GemmDType_F32) matmul_entry<float, false>(C, block, acc, A, RECT, B, RECT, a);
+    else if (dtype == FaerB200_GemmDType_C64) matmul_entry<double, true>(C, block, acc, A, RECT, B, RECT, a, conj_lhs, conj_rhs);
+    else matmul_entry<float, true>(C, block, acc, A, RECT, B, RECT, a, conj_lhs, conj_rhs);
     return;
   }
   FB_ASSERT(dtype == FaerB200_GemmDType_F64, "faer_b200_gemm: scatter indices / diagonal scaling are built for f64 only");
@@ -1562,15 +876,14 @@ void faer_b200_gemm(int dtype, int itype, int instr_set, size_t m, size_t n, siz
     dd = (const double*)dd_own;
     dstride = 1;
   }
-  const double a = read_scalar_f64((const FaerV0_24_Scalar*)alpha);
+  const double a = read_real<double>(alpha);
   FaerV0_24_MatMut C{dst, c_rows, c_cols, dst_rs, dst_cs};
   const bool keep_old = accum != 0 || row_idx || col_idx || block != (int)FaerV0_24_Block_Rectangular;
-  Mat c(C, keep_old, st);
-  Mat l(A, st), r(B, st);
+  StagedMat c = stage(C, sizeof(double), keep_old, st), l = stage(A, sizeof(double), st), r = stage(B, sizeof(double), st);
   if (m > 0 && n > 0)
-    spicy_matmul_f64(st, c.s.view<double>(), block, (const long long*)dri, (const long long*)dci, accum ? 1 : 0,
-                     l.s.view<const double>(), r.s.view<const double>(), dd, dstride, a);
-  finish_all(st, {&c.s, &l.s, &r.s});  // synchronises the stream: the host vectors above may go
+    spicy_matmul_f64(st, c.view<double>(), block, (const long long*)dri, (const long long*)dci, accum ? 1 : 0,
+                     l.view<const double>(), r.view<const double>(), dd, dstride, a);
+  finish_all(st, {&c, &l, &r});  // synchronises the stream: the host vectors above may go
   if (dri) ws_free(dri);
   if (dci) ws_free(dci);
   if (dd_own) ws_free(dd_own);

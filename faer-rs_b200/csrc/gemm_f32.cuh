@@ -35,11 +35,10 @@ void gemm_c32(cudaStream_t stream, VF dst, int dst_struct, int accum, VCF lhs, i
 void solve_lower_triangular_in_place_f32(cudaStream_t stream, VCF tril, bool unit, VF rhs);
 void solve_upper_triangular_in_place_f32(cudaStream_t stream, VCF triu, bool unit, VF rhs);
 
-// f32 LLT (llt.cu, instantiated for float): same contract as llt_cholesky_in_place_f64 / llt_solve_in_place_f64 (linalg_f64.cuh)
+// f32 LLT (llt.cu, instantiated for float): same contract as llt_cholesky_in_place_f64 (linalg_f64.cuh)
 struct LltResult;
 struct LltParams;
 LltResult llt_cholesky_in_place_f32(cudaStream_t stream, VF A, float reg_delta, float reg_eps, LltParams params);
-void llt_solve_in_place_f32(cudaStream_t stream, VCF L, VF rhs);
 
 // c32 triangular solves, LLT and partial-pivoting LU (cplx.cu, instantiated for float; same contracts as the _c64 functions in
 // linalg_f64.cuh); views in COMPLEX element units

@@ -76,11 +76,24 @@ size_t lu_partial_piv_in_place_f64(cudaStream_t stream, VD A, void* perm_fwd, vo
                                    PartialPivLuParams params);
 
 // ---- solves on top of the factors (solve_f64.cu; reference llt/solve.rs:12-35, lu/partial_pivoting/solve.rs:21-54) ----
-void permute_rows_in_place_f64(cudaStream_t stream, VD rhs, const long long* perm_fwd_host);
-void llt_solve_in_place_f64(cudaStream_t stream, VCD L, VD rhs);
-void lu_solve_in_place_f64(cudaStream_t stream, VCD L, VCD U, const long long* perm_fwd_host, VD rhs);
+// one complex element as the C ABI lays it out: (re, im), aligned like R only (faer's c64 / c32 guarantee no more), so that a
+// kernel moving it never emits a vector access that would need 2 * sizeof(R) alignment
+template <class R>
+struct ReIm {
+  R re, im;
+};
+// rhs[i, :] <- rhs[perm_fwd[i], :]; perm_fwd: HOST int64 array of rhs.nrows entries. E: double / float, or ReIm<double> /
+// ReIm<float> for a complex view (complex-unit strides on an R* base) reinterpreted as one of (re, im) elements
+template <class E>
+void permute_rows_in_place(cudaStream_t stream, View<E> rhs, const long long* perm_fwd_host);
+// T: double or float
+template <class T>
+void llt_solve_in_place(cudaStream_t stream, View<const T> L, View<T> rhs);
+template <class T>
+void lu_solve_in_place(cudaStream_t stream, View<const T> L, View<const T> U, const long long* perm_fwd_host, View<T> rhs);
 // rhs <- A^-T rhs (lu/partial_pivoting/solve.rs:55-86); perm_bwd: HOST int64 array, the inverse row permutation
-void lu_solve_transpose_in_place_f64(cudaStream_t stream, VCD L, VCD U, const long long* perm_bwd_host, VD rhs);
+template <class T>
+void lu_solve_transpose_in_place(cudaStream_t stream, View<const T> L, View<const T> U, const long long* perm_bwd_host, View<T> rhs);
 
 // workspace-based LU building blocks (used by dist.cu); all work is enqueued on the stream given at creation
 struct LuWorkspace;

@@ -272,10 +272,4 @@ LltResult llt_cholesky_in_place_f32(cudaStream_t stream, VF A, float reg_delta, 
   return llt_recursive_in_place<float>(stream, A, reg_delta, reg_eps, params);
 }
 
-void llt_solve_in_place_f32(cudaStream_t stream, VCF L, VF rhs) {
-  FB_ASSERT(L.nrows == L.ncols && rhs.nrows == L.nrows, "LLT solve shape mismatch");
-  solve_lower_triangular_in_place_f32(stream, L, false, rhs);
-  solve_upper_triangular_in_place_f32(stream, L.t(), false, rhs);
-}
-
 }  // namespace fb

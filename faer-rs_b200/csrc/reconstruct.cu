@@ -75,7 +75,7 @@ void lu_reconstruct_f64(cudaStream_t st, VD out, VCD L, VCD U, const long long* 
     gemm_f64(st, out.sub(0, size, size, n - size), RECT, 0, L.sub(0, 0, size, size), UNIT_LOWER, U.sub(0, size, size, n - size),
              RECT, 1.0);
   // (P A)[i, :] = A[perm_fwd[i], :]  =>  A[j, :] = (L U)[perm_bwd[j], :]
-  permute_rows_in_place_f64(st, out, perm_bwd);
+  permute_rows_in_place(st, out, perm_bwd);
 }
 
 void lu_inverse_f64(cudaStream_t st, VD out, VCD L, VCD U, const long long* perm_fwd) {
@@ -83,7 +83,7 @@ void lu_inverse_f64(cudaStream_t st, VD out, VCD L, VCD U, const long long* perm
   FB_ASSERT(out.ncols == n && L.nrows == n && L.ncols == n && U.nrows == n && U.ncols == n, "lu_inverse shape mismatch");
   if (n == 0) return;
   set_identity(st, out);
-  lu_solve_in_place_f64(st, L, U, perm_fwd, out);
+  lu_solve_in_place(st, L, U, perm_fwd, out);
 }
 
 template <class T>

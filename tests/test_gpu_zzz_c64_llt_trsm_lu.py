@@ -105,3 +105,33 @@ def test_c64_lu_vs_oracle(fb, oracle):
                     assert np.max(np.abs(Ae @ X - B)) <= 256 * n * U * np.linalg.cond(A) * np.max(np.abs(B)), (n, conj)
                     X = B.copy(order="F"); la.lu_solve_transpose_in_place(got, p, pi, X, conj)  # solve.rs:55-86
                     assert np.max(np.abs(Ae.T @ X - B)) <= 256 * n * U * np.linalg.cond(A) * np.max(np.abs(B)), (n, conj, "T")
+
+
+@pytest.mark.parametrize("cdt,rdt", [(np.complex128, np.float64), (np.complex64, np.float32)])
+def test_lu_solves_on_a_device_rhs_aligned_to_the_real_type(fb, cdt, rdt):
+    """faer's c64 / c32 are aligned like f64 / f32 only, so a device rhs may start at 8 mod 16 bytes (c64) or 4 mod 8 (c32). The
+    complex LU solves, row permutation included, use such a rhs in place and solve within the same backward bound as on the host."""
+    import torch
+    la, capi = fb.linalg, fb.capi
+    lib = capi.load()
+    rng = np.random.default_rng(7)
+    n, k = 300, 3
+    A = crandn(rng, (n, n)).astype(cdt)
+    LU = A.copy(order="F")
+    p = np.zeros(n, np.uint64); pi = np.zeros(n, np.uint64)
+    la.lu_in_place(LU, p, pi)
+    B = crandn(rng, (n, k)).astype(cdt)
+    suf = "c64" if cdt == np.complex128 else "c32"
+    u = U if cdt == np.complex128 else 2.0 ** -24
+    bound = 256 * n * u * np.linalg.cond(A.astype(np.complex128)) * np.max(np.abs(B))
+    for name, op in (("partial_piv_lu_solve_in_place", A), ("partial_piv_lu_solve_transpose_in_place", A.T)):
+        # one real element in front of the complex entries: the base is aligned to the real type and no more
+        buf = torch.zeros(1 + 2 * n * k, dtype=torch.float64 if rdt == np.float64 else torch.float32, device="cuda")
+        buf[1:] = torch.from_numpy(np.ascontiguousarray(B.T).view(rdt).reshape(-1)).cuda()
+        ptr = buf.data_ptr() + buf.element_size()
+        assert ptr % (2 * buf.element_size()) != 0
+        getattr(lib, f"libfaer_v0_23_{name}_u64_{suf}")(capi.mat_ref(LU), capi.mat_ref(LU), 0, capi.slice_mut(p), capi.slice_mut(pi),
+                                                       capi.MatMut(ptr, n, k, 1, n), capi.par_default(), capi.MemAlloc(None, 0))
+        torch.cuda.synchronize()
+        got = buf[1:].cpu().numpy().view(cdt).reshape(k, n).T
+        assert np.max(np.abs(op.astype(np.complex128) @ got.astype(np.complex128) - B)) <= bound, name
